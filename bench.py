@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] ...    # CPU baseline arm (oracle port)
+    python bench.py ... --dump-outputs DIR                         # also write the last timed step's outputs to DIR/*.npy
 
 One "step" = one cz_step launch advancing every environment of this rank once (each agent acts,
 rewards / termination / truncation computed, every agent's float64 feature vector written).
@@ -248,9 +249,8 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    # each "step" = every host core advances its own environment once; the timed sample is bounded on both sides:
-    # at least 2000 env-steps per core (a short --steps would time little more than noise), at most 60000 (minutes)
-    timed, warm = min(max(args.steps, 2000), 60000), min(max(args.warmup, 50), 2000)
+    # each "step" = every host core advances its own environment once
+    timed, warm = args.steps, args.warmup
     extra = {}
     if reference_available():
         kind = "reference"
@@ -391,6 +391,9 @@ def run_gpu_arm(args):
             dist.barrier()
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         env._bench_graph = graph        # keep the graph (and its captured pointers) alive as long as the environment
+        # the steps this environment took (warm-up, the graph's untimed replay, timed) and the steps per graph (0: eager
+        # launches): with a graph, step s of each replay takes actions[s % ring], so the last step's outputs depend on it
+        env._bench_schedule = (args.warmup, G if graph is not None else 0, K, G if graph is not None else 0)
         return env, float(t.item()), launches, clocks, how
 
     def timed_run_eager(pipelined, sample_clocks, obs_dtype):
@@ -422,6 +425,8 @@ def run_gpu_arm(args):
     except Exception as ex:
         bg_block = {"error": f"{type(ex).__name__}: {str(ex)[:160]}"}
     env, ms_total_max, launches, clocks, how_timed = timed_run(head_pipe, True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(env, args.dump_outputs)       # before the e2e leg below steps the same state further
     lib = env.lib
     ms_per_step = ms_total_max / args.steps
     value = world * N * args.steps / (ms_total_max / 1e3)
@@ -848,6 +853,34 @@ def run_gpu_arm(args):
         dist.destroy_process_group()
 
 
+DUMP_ENVS = 8192     # environments whose outputs --dump-outputs writes: 8192 x 2 agents x 278 f64 observations = 36 MB
+
+
+def dump_outputs(env, out_dir):
+    """What the last timed step returned to its caller (observations, rewards, terminated / truncated flags and the info
+    fields), as out_dir/<name>.npy, for a fixed seeded sample of DUMP_ENVS environments (every environment when there are
+    no more); env_index.npy lists the sampled environments.  Integer outputs are written as float32 (exact below 2**24).
+    schedule.npy holds how the environment got there: [warm-up steps, untimed graph steps, timed steps, steps per CUDA
+    graph (0: eager launches)]; two runs whose schedules differ (a graph capture that failed on one build) computed
+    different steps, and their outputs are not comparable."""
+    import torch
+    env.wait()
+    torch.cuda.synchronize(env.device)
+    N = env.num_envs
+    pick = np.arange(N) if N <= DUMP_ENVS else np.sort(np.random.default_rng(0).choice(N, DUMP_ENVS, replace=False))
+    idx = torch.from_numpy(pick).to(env.device)
+    info = env.info()
+    out = {"obs": env.obs, "reward": env.reward, "terminated": env.terminated, "truncated": env.truncated,
+           "info_t": info["t"], "info_done": info["done"], "info_recipe_done": info["recipe_done"],
+           "info_active": info["active"], "info_error_flags": info["error_flags"]}
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), pick.astype(np.float64))
+    np.save(os.path.join(out_dir, "schedule.npy"), np.array(env._bench_schedule, np.float64))
+    for name, t in out.items():
+        a = t[idx].cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype in (np.float64, np.float32) else a.astype(np.float32))
+
+
 _STDOUT_FD = None
 
 
@@ -877,7 +910,14 @@ def main():
                     help="sync (default, the headline): the in-place step (dynamics kernel, then the whole-row TMA writer, caller's "
                          "stream); pipelined: throughput mode for open-loop action streams, the dynamics of step k+1 run beside "
                          "the observation writes of step k (two kernels, two streams, ping-pong state, cz_pipeline_config)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one (a fixed sample of rank 0's environments) "
+                         "as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl cuda)")
     # stdout carries exactly one JSON line: everything libraries print while the run is under way (NCCL's version banner
     # goes to stdout when NCCL_DEBUG is set) is sent to stderr, and the descriptor is handed back for the final print
     sys.stdout.flush()
