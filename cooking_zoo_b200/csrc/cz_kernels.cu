@@ -1058,6 +1058,8 @@ struct cz_tables {
   uint64_t* h_layout_cum;   // host copy of the weighted pool's thresholds (cz_layout_index), or nullptr
   uint8_t* d_rand;          // scratch for device-generated actions outside the warp kernel
   int rand_envs;
+  void* d_keep;             // scratch rows of one step of a KEEP_ALL call whose per-step block is not 16-byte aligned
+  size_t keep_bytes;
   int num_sms;
   void* allocs[32];
   int n_allocs;
@@ -1370,6 +1372,7 @@ extern "C" int cz_tables_destroy(cz_tables* t) {
   if (t->d_term) cudaFree(t->d_term);
   if (t->d_trunc) cudaFree(t->d_trunc);
   if (t->d_rand) cudaFree(t->d_rand);
+  if (t->d_keep) cudaFree(t->d_keep);
   delete[] t->h_layout_cum;
   if (t->pipe_ready) {
     cudaStreamDestroy(t->pipe_dyn); cudaStreamDestroy(t->pipe_obs);
@@ -1717,9 +1720,24 @@ extern "C" int cz_step(const cz_tables* t, uint32_t* state, const uint8_t* actio
     }
     const size_t o = keep ? (size_t)k : 0;
     double* obs_k = obs ? reinterpret_cast<double*>(reinterpret_cast<char*>(obs) + o * obs_bytes) : nullptr;
+    // KEEP_ALL: step k's rows start k * obs_bytes into the buffer, which is 16-byte aligned only when obs_bytes is a multiple
+    // of 16 (odd n * A * L in float64, n * A * L not a multiple of 4 in float32); the row writers need 16-byte aligned rows,
+    // so such a step writes into aligned scratch that is then copied into place
+    double* dst = obs_k;
+    if (obs_k && ((uintptr_t)obs_k & 15) != 0) {
+      if (obs_bytes > t->keep_bytes) {
+        if (tm->d_keep) cudaFree(tm->d_keep);
+        tm->d_keep = nullptr;
+        tm->keep_bytes = 0;
+        CZ_CUDA(cudaMalloc(&tm->d_keep, obs_bytes));
+        tm->keep_bytes = obs_bytes;
+      }
+      obs_k = reinterpret_cast<double*>(tm->d_keep);
+    }
     int rc = cz_step_one(t, state, a, obs_k, reward + o * na, terminated + o * na, truncated + o * na, error_flags, n_envs,
                          flags & ~(CZ_STEP_DEVICE_ACTIONS | CZ_STEP_KEEP_ALL), seed, env_offset, stream);
     if (rc != CZ_OK) return rc;
+    if (dst != obs_k) CZ_CUDA(cudaMemcpyAsync(dst, obs_k, obs_bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   }
   return CZ_OK;
 }

@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 import torch
 
+from tests.kitchens import _random_level, _random_meta, _rich_level
 from tests.replay import ROOT
 
 pytestmark = pytest.mark.gpu
@@ -168,49 +169,12 @@ def test_single_steps_of_small_batches_take_the_warp_kernel_and_ragged_sizes_wor
         assert torch.equal(lane.state, warp.state)
 
 
-def _rich_level(rng, lp, mp):
-    """an 8x8 kitchen with many objects (more than 16 live dynamic slots: one environment per warp) and a meta file in
-    the order of example.json (packed observation plan: the specialised kernels)"""
-    import json
-    W = H = 8
-    rows = [["-"] * W] + [["-"] + [" "] * (W - 2) + ["-"] for _ in range(H - 2)] + [["-"] * W]
-    ring = [(x, 0) for x in range(1, W - 1)] + [(x, H - 1) for x in range(1, W - 1)] + \
-           [(0, y) for y in range(1, H - 1)] + [(W - 1, y) for y in range(1, H - 1)]
-    rng.shuffle(ring)
-    statics, need = [], {}
-    for name, count in (("Cutboard", 2), ("Blender", 1), ("Deliversquare", 2)):
-        for _ in range(count):
-            x, y = ring.pop()
-            statics.append({name: {"COUNT": 1, "X_POSITION": [x], "Y_POSITION": [y]}})
-            need[name] = need.get(name, 0) + 1
-    dyn = []
-    for name in ["Plate", "Tomato", "Onion", "Lettuce", "Carrot", "Banana", "Apple", "Watermelon", "Bread"]:
-        for _ in range(rng.randint(1, 3)):
-            if not ring:
-                break
-            x, y = ring.pop()
-            dyn.append({name: {"COUNT": 1, "X_POSITION": [x], "Y_POSITION": [y]}})
-            need[name] = need.get(name, 0) + 1
-    level = {"LEVEL_LAYOUT": "\n".join("".join(r) for r in rows), "STATIC_OBJECTS": statics, "DYNAMIC_OBJECTS": dyn,
-             "AGENTS": [{"MAX_COUNT": 4, "X_POSITION": list(range(1, W - 1)), "Y_POSITION": list(range(1, H - 1))}],
-             "DYNAMIC_EXCLUDED_POSITIONS": []}
-    json.dump(level, open(lp, "w"))
-    meta = []
-    for name in ["Cutboard", "Counter", "Blender", "Deliversquare", "Plate", "Tomato", "Onion", "Lettuce", "Carrot", "Banana",
-                 "Apple", "Watermelon", "Bread", "Agent", "Block", "Switch"]:
-        n = need.get(name, 0) + rng.randint(0, 1) + (need.get(name, 0) if name == "Bread" else 0)
-        n_counters = 2 * W + 2 * (H - 2) - sum(need.get(k, 0) for k in ("Cutboard", "Blender", "Deliversquare"))
-        meta.append({name: n_counters + rng.randint(0, 1) if name == "Counter" else (4 if name == "Agent" else n)})
-    json.dump(meta, open(mp, "w"))
-
-
 def test_k_steps_on_random_levels_and_meta_files(tmp_path, monkeypatch):
     """the property-test generator of tests/test_oracle_vs_reference.py (random open kitchens up to 8x8, random meta
     counts and order, OPTIONAL objects, 1-4 agents, both action schemes, despawn / respawn): K steps in one launch of the
     warp kernel against K launches of the lane kernels, table classes and group widths as they fall"""
     import random
     from cooking_zoo_b200 import BatchedCookingEnv
-    from tests.test_oracle_vs_reference import _random_level, _random_meta
     widths = set()
     for seed in range(5000, 5024):
         rng = random.Random(seed)

@@ -9,7 +9,8 @@ import torch
 
 from oracle.cz_oracle import RECIPES, SpawnStream
 from tests.replay import assert_state_equal, assert_obs_equal, bits, ROOT
-from tests.test_oracle_vs_reference import _random_level, _random_meta, OPEN4, META4
+from tests.kitchens import _random_level, _random_meta
+from tests.test_oracle_vs_reference import OPEN4, META4
 
 pytestmark = [pytest.mark.gpu, pytest.mark.reference]
 BOOK = list(RECIPES)

@@ -388,8 +388,7 @@ def test_generic_tables_large_batch_any_plan_writer(monkeypatch, tmp_path):
     (more than 64 pairs, long table runs, odd row lengths)."""
     import random
     from cooking_zoo_b200 import BatchedCookingEnv
-    from tests.test_oracle_vs_reference import _random_level, _random_meta
-    from tests.test_gpu_ksteps import _rich_level
+    from tests.kitchens import _random_level, _random_meta, _rich_level
     cfg = dict(level="coop_test", meta_file="example", num_agents=2, max_steps=30,
                recipes=["TomatoLettuceSalad", "CarrotBanana"], end_all=True, reward_scheme=None)
     n = 50001

@@ -2,7 +2,6 @@
 action schemes, despawn / respawn, 1-4 agents, plus property tests over random meta counts and random open levels.
 Runs wherever the reference is importable: /root/reference in the build container, the verbatim copy in oracle/_ref
 (python -m oracle.make_ref) on the GPU box."""
-import json
 import os
 import random
 
@@ -11,6 +10,7 @@ import pytest
 
 from oracle.cz_oracle import OracleEnv, RECIPES, SpawnStream
 from oracle.cz_oracle_c import COracleEnv
+from tests.kitchens import _random_level, _random_meta
 from tests.replay import assert_state_equal, assert_obs_equal, bits, ROOT
 
 pytestmark = pytest.mark.reference
@@ -92,57 +92,6 @@ def test_live_lockstep_one_to_four_agents_with_despawn_and_respawn(level, A):
 
 
 # ---- property tests: random meta counts, random open levels (at most 8x8), random action streams -------------------
-def _random_level(rng, path):
-    """an open kitchen: counter ring, random inner counters, appliances on the ring, ingredients on counters"""
-    W, H = rng.randint(5, 8), rng.randint(5, 8)
-    rows = [["-"] * W] + [["-"] + [" "] * (W - 2) + ["-"] for _ in range(H - 2)] + [["-"] * W]
-    for _ in range(rng.randint(0, 3)):
-        rows[rng.randint(2, H - 3)][rng.randint(2, W - 3)] = "-"
-    ring = [(x, 0) for x in range(1, W - 1)] + [(x, H - 1) for x in range(1, W - 1)] + \
-           [(0, y) for y in range(1, H - 1)] + [(W - 1, y) for y in range(1, H - 1)]
-    rng.shuffle(ring)
-    statics = []
-    for name, count in (("Cutboard", rng.randint(1, 2)), ("Blender", rng.randint(0, 1)), ("Deliversquare", rng.randint(1, 2))):
-        for _ in range(count):
-            x, y = ring.pop()
-            statics.append({name: {"COUNT": 1, "X_POSITION": [x], "Y_POSITION": [y]}})
-    foods = ["Plate", "Plate", "Tomato", "Lettuce", "Carrot", "Banana", "Bread", "Onion", "Apple", "Watermelon"]
-    rng.shuffle(foods)
-    dyn = []
-    for name in foods[:rng.randint(3, 8)]:
-        x, y = ring.pop()          # one cell per entry: a cross product of two ring cells could name a taken or a floor cell
-        entry = {"COUNT": 1, "X_POSITION": [x], "Y_POSITION": [y]}
-        if rng.random() < 0.2:
-            entry["OPTIONAL"] = 0.5
-        dyn.append({name: entry})
-    agents = [{"MAX_COUNT": 2, "X_POSITION": list(range(1, W - 1)), "Y_POSITION": list(range(1, H - 1))},
-              {"MAX_COUNT": 2, "X_POSITION": list(range(1, W - 1)), "Y_POSITION": list(range(1, H - 1))}]
-    level = {"LEVEL_LAYOUT": "\n".join("".join(r) for r in rows), "STATIC_OBJECTS": statics, "DYNAMIC_OBJECTS": dyn,
-             "AGENTS": agents, "DYNAMIC_EXCLUDED_POSITIONS": []}
-    json.dump(level, open(path, "w"))
-    return level
-
-
-def _random_meta(rng, level, path):
-    need = {}
-    for group in ("STATIC_OBJECTS", "DYNAMIC_OBJECTS"):
-        for entry in level[group]:
-            (name, spec), = entry.items()
-            need[name] = need.get(name, 0) + spec["COUNT"]
-    order = ["Cutboard", "Counter", "Blender", "Deliversquare", "Plate", "Tomato", "Onion", "Lettuce", "Carrot", "Banana",
-             "Apple", "Watermelon", "Bread", "Agent", "Block", "Switch"]
-    rng.shuffle(order)
-    meta = []
-    for name in order:
-        lo = need.get(name, 0) + (1 if name == "Bread" and need.get(name, 0) else 0)       # room for a chopped twin
-        if name == "Counter":
-            lo = 64
-        if name == "Agent":
-            lo = 4
-        meta.append({name: lo + rng.randint(0, 2)})
-    json.dump(meta, open(path, "w"))
-
-
 def test_property_random_levels_and_meta_files(tmp_path):
     hyp = pytest.importorskip("hypothesis")
     from hypothesis import given, settings, strategies as st, HealthCheck

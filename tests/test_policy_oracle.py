@@ -51,12 +51,20 @@ def test_policy_goldens_cover_crashes_and_all_moves():
 @pytest.mark.parametrize("level,meta,agents", [("coop_test", "example", 2), ("switch_test", "example", 2),
                                                ("coexistence_test", "example", 2),
                                                ("tests/golden/levels/open4.json", "tests/golden/levels/meta4.json", 4),
-                                               ("tests/golden/levels/tiny4.json", "tests/golden/levels/meta4.json", 4)])
-def test_policy_tables_match_the_queue_level_searches(level, meta, agents):
+                                               ("tests/golden/levels/tiny4.json", "tests/golden/levels/meta4.json", 4),
+                                               # kitchen_<seed>: tests/kitchens.kitchen(seed), meta file included; seeds
+                                               # 1, 5, 9 and 13 are split in two by an inner wall, 4 is a rich kitchen
+                                               ("kitchen_1", None, 2), ("kitchen_5", None, 4), ("kitchen_9", None, 1),
+                                               ("kitchen_13", None, 3), ("kitchen_2", None, 2), ("kitchen_7", None, 3),
+                                               ("kitchen_4", None, 2)])
+def test_policy_tables_match_the_queue_level_searches(level, meta, agents, tmp_path):
     """reach / first_step / lists of cooking_zoo_b200/policy.py == oracle.cz_policy.reachable / walk on every cell pair"""
     from cooking_zoo_b200.tables import compile_tables, ROW_VARIANT
     from cooking_zoo_b200.policy import compile_policy_tables
+    from tests.kitchens import kitchen
     from tests.replay import ROOT
+    if level.startswith("kitchen_"):
+        level, meta, _ = kitchen(int(level[len("kitchen_"):]), str(tmp_path))
     path = lambda p: os.path.join(ROOT, p) if p.endswith(".json") else p
     t = compile_tables(path(level), path(meta), agents, 100, ["TomatoSalad"] * agents, layout_pool_size=24, layout_seed=5)
     p = compile_policy_tables(t)
