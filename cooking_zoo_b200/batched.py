@@ -15,6 +15,7 @@ import torch
 
 from . import _native
 from .tables import compile_tables, NUM_MISC, ROW_SBITS, ROW_TINFO, ROW_MARKS, ROW_VARIANT
+from .grid import grid_channels
 
 
 _ALWAYS_GUARD = os.environ.get("CZ_PY_DEVICE_GUARD") == "1"   # A/B: always enter torch.cuda.device(...) around library calls
@@ -47,9 +48,18 @@ class BatchedCookingEnv:
                  auto_reset=False, seed=0, env_offset=0, pipelined=False, obs_dtype=torch.float64, stream=None,
                  pipeline_buffers=2, background_dynamics=0, background_policy=0):
         obs_spaces = obs_spaces or ["feature_vector"] * num_agents
-        if any(o != "feature_vector" for o in obs_spaces):
-            raise NotImplementedError("the batched entry point builds feature_vector observations only "
-                                      "(symbolic/full are host object graphs in the reference)")
+        if obs_spaces and all(o == "grid" for o in obs_spaces):
+            # per-cell u8 planes [N, A, C, H, W] written by their own kernel after the dynamics (cooking_zoo_b200.grid)
+            if pipelined:
+                raise NotImplementedError("the pipelined step writes feature_vector observations only")
+            if obs_dtype != torch.float64:
+                raise ValueError("obs_dtype applies to feature_vector observations; the grid is uint8")
+            self.obs_mode = "grid"
+        elif any(o != "feature_vector" for o in obs_spaces):
+            raise NotImplementedError("the batched entry point builds feature_vector or grid observations, the same "
+                                      "kind for every agent (symbolic/full are host object graphs in the reference)")
+        else:
+            self.obs_mode = "feature_vector"
         if action_scheme not in ("scheme1", "scheme3"):
             raise NotImplementedError("action_scheme must be 'scheme1' or 'scheme3' (scheme2 raises AttributeError "
                                       "in the reference itself, action_scheme2.py:15)")
@@ -92,7 +102,16 @@ class BatchedCookingEnv:
         self.obs_dtype = obs_dtype
         self._flags = (_native.STEP_AUTO_RESET if self.auto_reset else 0) | \
                       (_native.STEP_OBS_F32 if obs_dtype == torch.float32 else 0)
-        self.obs = torch.zeros((N, A, L), dtype=obs_dtype, device=dev)
+        self.grid_channels = grid_channels(t)
+        if self.lib.cz_grid_channels(self._handle) != len(self.grid_channels):
+            raise _native.NativeError("libcz_b200.so and cooking_zoo_b200.grid disagree on the grid's channels")
+        self._grid_shape = (N, A, len(self.grid_channels), t.height, t.width)
+        if self.obs_mode == "grid":
+            self.obs = torch.zeros(self._grid_shape, dtype=torch.uint8, device=dev)
+            # chosen once here, so that the feature-vector methods keep their host code unchanged
+            self.__class__ = _GridModeEnv
+        else:
+            self.obs = torch.zeros((N, A, L), dtype=obs_dtype, device=dev)
         self.reward = torch.zeros((N, A), dtype=torch.float64, device=dev)
         self.terminated = torch.zeros((N, A), dtype=torch.uint8, device=dev)
         self.truncated = torch.zeros((N, A), dtype=torch.uint8, device=dev)
@@ -167,6 +186,7 @@ class BatchedCookingEnv:
             mk = torch.as_tensor(mask).to(torch.uint8).to(self.device).contiguous()
         with torch.cuda.device(self.device):
             f32 = self.obs_dtype == torch.float32
+            grid = self.obs_mode == "grid"
             if self.pipelined:
                 # drain the internal streams (dynamics / row writer still in flight) and keep stepping from the half
                 # that holds the current state: a masked reset must land next to the untouched environments
@@ -176,8 +196,11 @@ class BatchedCookingEnv:
             _native.check(self.lib.cz_reset(self._handle, self.state.data_ptr(), lid.data_ptr(),
                                             rid.data_ptr() if rid is not None else None,
                                             mk.data_ptr() if mk is not None else None,
-                                            None if f32 else self.obs.data_ptr(), self.error_flags.data_ptr(), N,
-                                            self._stream()))
+                                            None if f32 or grid else self.obs.data_ptr(), self.error_flags.data_ptr(),
+                                            N, self._stream()))
+            if grid:
+                _native.check(self.lib.cz_observe_grid(self._handle, self.state.data_ptr(), self.obs.data_ptr(), N,
+                                                       self._stream()))
             if f32:
                 _native.check(self.lib.cz_observe_f32(self._handle, self.state.data_ptr(), self.obs.data_ptr(), N,
                                                       self._stream()))
@@ -236,6 +259,76 @@ class BatchedCookingEnv:
                                            term.data_ptr(), trunc.data_ptr(), self.error_flags.data_ptr(), N, K, flags,
                                            self.seed, self.env_offset, int(action_step), self._stream()))
         return obs, rew, term, trunc, self._info
+
+    def _step_grid(self, actions):
+        """step() of grid mode: the dynamics (cz_step without observation rows), then the grid writer.
+        Returns (obs u8 [N, A, C, H, W], reward, terminated, truncated, info)."""
+        a = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions))
+        if a.shape != self._shape_actions:
+            raise ValueError("actions must have shape [num_envs, num_agents]")
+        if a.dtype != torch.uint8 or a.device != self.device or not a.is_contiguous():
+            self._actions.copy_(a)
+            a = self._actions
+        s = self._stream()
+        self._call(self.lib.cz_step, self._handle, self.state.data_ptr(), a.data_ptr(), None, self.reward.data_ptr(),
+                   self.terminated.data_ptr(), self.truncated.data_ptr(), self.error_flags.data_ptr(), self.num_envs, 1,
+                   self._flags, self.seed, self.env_offset, 0, s)
+        self._call(self.lib.cz_observe_grid, self._handle, self.state.data_ptr(), self.obs.data_ptr(), self.num_envs, s)
+        return self.obs, self.reward, self.terminated, self.truncated, self._info
+
+    def _step_k_grid(self, k_steps, actions=None, action_step=0, keep_all=False):
+        """step_k() of grid mode.  keep_all=False: one cz_step of k_steps without observation rows, then one grid write.
+        keep_all=True: k single steps, each followed by its grid write into a fresh [k_steps, N, A, C, H, W] tensor."""
+        N, A, K = self.num_envs, self.num_agents, int(k_steps)
+        flags = self._flags
+        if actions is None:
+            flags |= _native.STEP_DEVICE_ACTIONS
+        else:
+            a = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions))
+            if a.shape != (K, N, A):
+                raise ValueError("actions must have shape [k_steps, num_envs, num_agents]")
+            a = a.to(device=self.device, dtype=torch.uint8).contiguous()
+            self._k_actions = a          # keep alive until the launch has consumed it
+        s = self._stream()
+        with torch.cuda.device(self.device):
+            if not keep_all:
+                _native.check(self.lib.cz_step(self._handle, self.state.data_ptr(), None if actions is None else a.data_ptr(),
+                                               None, self.reward.data_ptr(), self.terminated.data_ptr(),
+                                               self.truncated.data_ptr(), self.error_flags.data_ptr(), N, K, flags, self.seed,
+                                               self.env_offset, int(action_step), s))
+                _native.check(self.lib.cz_observe_grid(self._handle, self.state.data_ptr(), self.obs.data_ptr(), N, s))
+                return self.obs, self.reward, self.terminated, self.truncated, self._info
+            obs = torch.empty((K,) + self._grid_shape, dtype=torch.uint8, device=self.device)
+            rew = torch.empty((K, N, A), dtype=torch.float64, device=self.device)
+            term = torch.empty((K, N, A), dtype=torch.uint8, device=self.device)
+            trunc = torch.empty((K, N, A), dtype=torch.uint8, device=self.device)
+            for j in range(K):
+                _native.check(self.lib.cz_step(self._handle, self.state.data_ptr(),
+                                               None if actions is None else a[j].data_ptr(), None, rew[j].data_ptr(),
+                                               term[j].data_ptr(), trunc[j].data_ptr(), self.error_flags.data_ptr(), N, 1,
+                                               flags, self.seed, self.env_offset, int(action_step) + j, s))
+                _native.check(self.lib.cz_observe_grid(self._handle, self.state.data_ptr(), obs[j].data_ptr(), N, s))
+        return obs, rew, term, trunc, self._info
+
+    def _observe_grid(self):
+        with torch.cuda.device(self.device):
+            _native.check(self.lib.cz_observe_grid(self._handle, self.state.data_ptr(), self.obs.data_ptr(),
+                                                   self.num_envs, self._stream()))
+        return self.obs
+
+    def grid_observation(self, out=None):
+        """The grid observation of the current state, in either observation mode: uint8 [N, A, C, H, W] with the channels
+        named by grid_channels (cooking_zoo_b200.grid; cell (x, y) at [..., y, x]).  out: a contiguous uint8 tensor of
+        that shape on this device (any byte offset), or None for a new tensor."""
+        if out is None:
+            out = torch.empty(self._grid_shape, dtype=torch.uint8, device=self.device)
+        elif (tuple(out.shape) != self._grid_shape or out.dtype != torch.uint8 or out.device != self.device
+              or not out.is_contiguous()):
+            raise ValueError(f"out must be a contiguous uint8 tensor of shape {self._grid_shape} on {self.device}")
+        with torch.cuda.device(self.device):
+            _native.check(self.lib.cz_observe_grid(self._handle, self.state.data_ptr(), out.data_ptr(), self.num_envs,
+                                                   self._stream()))
+        return out
 
     def _step_pipelined(self, a):
         self._call(self.lib.cz_step_pipelined, self._handle, self._state2.data_ptr(), a.data_ptr(), self.obs.data_ptr(),
@@ -468,3 +561,10 @@ class BatchedCookingEnv:
                 if r >> 6 & 1 and (r >> 10) & 3 == 2 and (r >> 12) & 31 == h:
                     col[s] = (r & ~63) | xy
         self.state[:, env] = torch.from_numpy(col.astype(np.int32)).to(self.device)
+
+
+class _GridModeEnv(BatchedCookingEnv):
+    """A BatchedCookingEnv constructed with obs_spaces=["grid"] * num_agents: step / step_k / observe write the grid."""
+    step = BatchedCookingEnv._step_grid
+    step_k = BatchedCookingEnv._step_k_grid
+    observe = BatchedCookingEnv._observe_grid

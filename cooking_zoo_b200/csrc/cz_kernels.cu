@@ -1029,6 +1029,8 @@ cz_obs_any_whole_kernel(const __grid_constant__ CzDev T, const uint32_t* __restr
   }
 }
 
+#include "cz_grid.cuh"
+
 // =========================================================================================
 // Host side: tables object and the C ABI
 // =========================================================================================
@@ -1084,6 +1086,7 @@ struct cz_tables {
   int pipe_dyn_blocks;   // blocks per SM the dynamics kernel of the pipelined step is launched with (0 = no cap): a small grid that
                          // loops over its tiles runs in the background of the row writer instead of displacing it
   size_t smem_optin;
+  CzGridDev grid;           // the grid observation writer's constants (cz_grid.cuh)
 };
 
 template <typename Tp>
@@ -1294,6 +1297,27 @@ extern "C" int cz_tables_create(const cz_table_desc* d, int device, cz_tables** 
     const unsigned char* dimg = nullptr;
     rc = upload(t, img_buf, img_bytes, &dimg);
     T.blob = dimg;
+  }
+  if (rc == CZ_OK) {  // grid observation: channel numbers of every dynamic slot (channel order in cz_b200.h)
+    CzGridDev& g = t->grid;
+    int n_chop = 0, n_mash = 0;
+    for (int i = 0; i < T.T; ++i) {
+      n_chop += (d->type_flags[i] & 2) != 0;
+      n_mash += (d->type_flags[i] & 4) != 0;
+    }
+    uint32_t type_ch[CZ_MAX_TYPES], slot_ch[CZ_MAX_DYN];
+    for (int i = 0, kc = 0, km = 0; i < T.T; ++i) {
+      const uint32_t chop = (d->type_flags[i] & 2) ? (uint32_t)(12 + T.T + kc++) : 0u;
+      const uint32_t mash = (d->type_flags[i] & 4) ? (uint32_t)(12 + T.T + n_chop + km++) : 0u;
+      type_ch[i] = (uint32_t)(12 + i) | chop << 8 | mash << 16;
+    }
+    for (int s = 0; s < T.D; ++s) slot_ch[s] = d->slot_type[s] < T.T ? type_ch[d->slot_type[s]] : 0u;
+    g.W = T.W; g.H = T.H; g.HW = T.W * T.H; g.D = T.D; g.rows = T.rows;
+    g.G0 = 12 + T.T + n_chop + n_mash + 1;
+    g.C = g.G0 + 7 * T.A;
+    g.E = (uint32_t)(T.A * g.C * g.HW);
+    g.grid = T.grid;
+    rc = upload(t, slot_ch, T.D, &g.slot_ch);
   }
   if (rc != CZ_OK) { cz_tables_destroy(t); return rc; }
   size_t smem = cz_smem_bytes(T);
@@ -1753,6 +1777,32 @@ extern "C" int cz_observe(const cz_tables* t, const uint32_t* state, double* obs
     return cz_launch_obs_any(t, state, obs, n_envs, (cudaStream_t)stream);
   return cz_launch<MODE_OBSERVE>(t, state, const_cast<uint32_t*>(state), false, nullptr, nullptr, nullptr, nullptr, obs, nullptr,
                                  nullptr, nullptr, nullptr, n_envs, 0, 0, 0, stream);
+}
+
+extern "C" int cz_grid_channels(const cz_tables* t) {
+  if (!t) return cz_fail(CZ_EINVAL, "%s", "null argument");
+  return t->grid.C;
+}
+
+extern "C" int cz_observe_grid(const cz_tables* t, const uint32_t* state, uint8_t* grid, int n_envs, void* stream) {
+  if (!t || !state || !grid) return cz_fail(CZ_EINVAL, "%s", "null argument");
+  if (n_envs <= 0) return CZ_OK;
+  const CzGridDev& G = t->grid;
+  int warps = (int)(GRID_SMEM_BUDGET / G.E);  // E <= 4 agents x 89 channels x 64 cells = 22784 bytes: at least one
+  if (warps > GRID_WARPS) warps = GRID_WARPS;
+  if (warps < 1) warps = 1;
+  const size_t smem = ((size_t)warps * G.E + 30) & ~(size_t)15;  // up to 15 bytes of shift in front, rounded up to 16
+  const int blocks = (n_envs + warps - 1) / warps;
+  cudaStream_t s = (cudaStream_t)stream;
+  switch (t->dev.A) {
+    case 1: cz_grid_kernel<1><<<blocks, 32 * warps, smem, s>>>(G, state, grid, n_envs, warps); break;
+    case 2: cz_grid_kernel<2><<<blocks, 32 * warps, smem, s>>>(G, state, grid, n_envs, warps); break;
+    case 3: cz_grid_kernel<3><<<blocks, 32 * warps, smem, s>>>(G, state, grid, n_envs, warps); break;
+    default: cz_grid_kernel<4><<<blocks, 32 * warps, smem, s>>>(G, state, grid, n_envs, warps); break;
+  }
+  g_launches.fetch_add(1);
+  CZ_CUDA(cudaGetLastError());
+  return CZ_OK;
 }
 
 static int cz_pipe_init(cz_tables* t) {

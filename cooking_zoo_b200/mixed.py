@@ -18,6 +18,9 @@ from .batched import BatchedCookingEnv
 class MixedAgentCookingEnv:
     def __init__(self, agent_counts, level, meta_file, max_steps, recipes, *, device="cuda:0", env_offset=0,
                  layouts_by_count=None, **kwargs):
+        if any(o == "grid" for o in kwargs.get("obs_spaces") or ()):
+            # the grid's channel count grows with the agent count: the groups would not share one observation shape
+            raise NotImplementedError("MixedAgentCookingEnv builds feature_vector observations only")
         counts = np.asarray(agent_counts, dtype=np.int64)
         if counts.ndim != 1 or counts.size == 0 or counts.min() < 1:
             raise ValueError("agent_counts must be a non-empty vector of positive agent counts")

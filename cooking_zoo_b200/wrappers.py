@@ -36,8 +36,8 @@ class _Discrete:
     n: int
 
 
-def _box(low, high, shape):
-    return _gym.spaces.Box(low=low, high=high, shape=shape) if _gym else _Box(low, high, shape)
+def _box(low, high, shape, dtype=np.float32):
+    return _gym.spaces.Box(low=low, high=high, shape=shape, dtype=dtype) if _gym else _Box(low, high, shape, dtype)
 
 
 def _discrete(n):
@@ -65,8 +65,12 @@ class ParallelCookingEnv:
         book = list(active_book().keys())
         # quirk C-7 (cooking_env.py:155-161): agent i's goal vector is one-hot(i) over the book
         self.goal_vectors = {a: np.eye(len(book))[i] for i, a in enumerate(self.possible_agents)}
-        L = self._b.obs_len
-        self.observation_spaces = {a: _box(-1, 1, (L,)) for a in self.possible_agents}
+        if self._b.obs_mode == "grid":    # per-cell u8 planes [C, H, W] of the agent's world (cooking_zoo_b200.grid)
+            shape = (len(self._b.grid_channels), self._b.tables.height, self._b.tables.width)
+            self.observation_spaces = {a: _box(0, 255, shape, np.uint8) for a in self.possible_agents}
+        else:
+            L = self._b.obs_len
+            self.observation_spaces = {a: _box(-1, 1, (L,)) for a in self.possible_agents}
         self.action_spaces = {a: _discrete(self._b.tables.num_actions) for a in self.possible_agents}  # cooking_env.py:131
 
     def observation_space(self, agent):

@@ -195,6 +195,28 @@ int cz_observe(const cz_tables* t, const uint32_t* state, double* obs, int n_env
  * pays for float64 rows: cz_reset(..., NULL, ...) + cz_observe_f32, then cz_step with CZ_STEP_OBS_F32. */
 int cz_observe_f32(const cz_tables* t, const uint32_t* state, float* obs32, int n_envs, void* stream);
 
+/* ---- grid observation ----------------------------------------------------------------------
+ * Per-cell u8 planes of every agent's world: grid u8 [n][A][C][H][W], cell (x, y) at [..., y, x].  A pure function of the
+ * packed state (written after cz_reset / cz_step with obs == NULL) that does not depend on the observation plan.  C depends
+ * only on the meta file and A.  Channel order for observer a:
+ *   [0, 7)   static kinds in ST_* code order: floor, counter, cutboard, blender, deliversquare, switch, block.  1 where that
+ *            static stands; floor is every cell of the W x H grid where no other static stands (one-hot on every cell)
+ *   [7, 12)  cutboard_ready, blender_ready, blender_on, switch_active, block_walkable: 1 on the static's cell when its SBITS
+ *            bit is set
+ *   12 + t   n:<Type> for each dynamic type t of the meta file, in meta order (also types without device slots): number of
+ *            present objects of the type at the cell, held objects and plate contents included
+ *   then     chopped:<Type> for each type with the chop flag, in meta order: how many of them are chopped
+ *   then     mashed:<Type> for each type with the blend flag, in meta order: how many of them are mashed
+ *   then     on_plate: number of present objects at the cell whose container is a plate (container kind 2)
+ *   then     A agent groups g (group 0 = agent a, then the other agents in ascending index), 7 channels each:
+ *            agent<g> (position), agent<g>_facing1..4 (orientation 1..4), agent<g>_holding, agent<g>_active; 1 at the agent's
+ *            cell.  An inactive agent keeps its position and facing planes.
+ * So C = 7 + 5 + T + T_chop + T_blend + 1 + 7 A (46 for the shipped meta with two agents).  Not encoded: the order of
+ * contents, free flags, grace periods, the clock and recipe marks. */
+int cz_grid_channels(const cz_tables* t);
+/* grid of every environment from the current state, asynchronous on `stream`; no alignment requirement on `grid`. */
+int cz_observe_grid(const cz_tables* t, const uint32_t* state, uint8_t* grid, int n_envs, void* stream);
+
 /* The reference-facing call with HOST buffers: copies actions host->device, steps, copies
  * obs/reward/flags device->host, and synchronises the stream before returning.  Scratch
  * device buffers are owned by the tables object (sized on first use). */
