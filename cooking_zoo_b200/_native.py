@@ -16,6 +16,7 @@ STEP_AUTO_RESET = 1
 STEP_OBS_F32 = 2
 STEP_DEVICE_ACTIONS = 4
 STEP_KEEP_ALL = 8
+STEP_EPISODE_STATS = 16
 ERR_BITS = {1: "CUTBOARD_NONE", 2: "REMOVE", 4: "SWITCH_LINK", 8: "SPAWN_LOC", 16: "TRUNC_DESPAWN", 32: "OBS_OVERFLOW",
             64: "OFFGRID", 128: "BAD_ID"}
 
@@ -44,6 +45,11 @@ class PolicyDesc(C.Structure):
                 ("reach", _P), ("first_step", _P)]
 
 
+class StatsDesc(C.Structure):
+    _fields_ = [("n_envs", C.c_int32)] + [(n, _P) for n in ("ret", "episode", "open", "last_ret", "last_len", "last_served",
+                                                            "last_success", "finished", "totals")]
+
+
 # every symbol include/cz_b200.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "cz_abi_version": (C.c_int, []),
@@ -59,6 +65,8 @@ SIGNATURES = {
     "cz_layout_ids": (C.c_int, [_P, _P, C.c_int, C.c_uint64, C.c_int64, C.c_uint64, _P]),
     "cz_step": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_uint32, C.c_uint64, C.c_int64,
                           C.c_uint64, _P]),
+    "cz_stats_attach": (C.c_int, [_P, C.POINTER(StatsDesc)]),
+    "cz_stats_clear": (C.c_int, [_P, _P, C.c_int, _P]),
     "cz_observe": (C.c_int, [_P, _P, _P, C.c_int, _P]),
     "cz_observe_f32": (C.c_int, [_P, _P, _P, C.c_int, _P]),
     "cz_grid_channels": (C.c_int, [_P]),

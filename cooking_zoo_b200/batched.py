@@ -46,7 +46,7 @@ class BatchedCookingEnv:
                  reward_scheme=None, agent_respawn_rate=0.0, grace_period=20, agent_despawn_rate=0.0, *,
                  device="cuda:0", recipe_pool=None, layout_pool_size="auto", layout_seed=0, layouts=None,
                  auto_reset=False, seed=0, env_offset=0, pipelined=False, obs_dtype=torch.float64, stream=None,
-                 pipeline_buffers=2, background_dynamics=0, background_policy=0):
+                 pipeline_buffers=2, background_dynamics=0, background_policy=0, episode_stats=False):
         obs_spaces = obs_spaces or ["feature_vector"] * num_agents
         if obs_spaces and all(o == "grid" for o in obs_spaces):
             # per-cell u8 planes [N, A, C, H, W] written by their own kernel after the dynamics (cooking_zoo_b200.grid)
@@ -120,6 +120,35 @@ class BatchedCookingEnv:
         self._info = _LazyInfo(self)
         self._dev_index = dev.index if dev.index is not None else torch.cuda.current_device()
         self._shape_actions = (N, A)
+        self._stats = None
+        if episode_stats:
+            self._attach_episode_stats()
+
+    def _attach_episode_stats(self):
+        """episode statistics on the device (cz_stats_attach): every step path updates them from here on"""
+        N, A, dev = self.num_envs, self.num_agents, self.device
+        st = {"return": torch.zeros((N, A), dtype=torch.float64, device=dev),
+              "episode": torch.zeros((N,), dtype=torch.int32, device=dev),      # u32 bits of the EPISODE row last seen
+              "open": torch.zeros((N,), dtype=torch.uint8, device=dev),
+              "last_return": torch.zeros((N, A), dtype=torch.float64, device=dev),
+              "last_length": torch.zeros((N,), dtype=torch.int32, device=dev),
+              "last_served": torch.zeros((N,), dtype=torch.uint8, device=dev),
+              "last_success": torch.zeros((N,), dtype=torch.uint8, device=dev),
+              "finished": torch.zeros((N,), dtype=torch.int32, device=dev),
+              "totals": torch.zeros((4 + A,), dtype=torch.float64, device=dev)}
+        d = _native.StatsDesc()
+        d.n_envs = N
+        for field, key in (("ret", "return"), ("episode", "episode"), ("open", "open"), ("last_ret", "last_return"),
+                           ("last_len", "last_length"), ("last_served", "last_served"), ("last_success", "last_success"),
+                           ("finished", "finished"), ("totals", "totals")):
+            setattr(d, field, st[key].data_ptr())
+        with torch.cuda.device(dev):
+            _native.check(self.lib.cz_stats_attach(self._handle, C.byref(d)))
+        self._stats = st
+        self.episode_totals_names = ["episodes", "length", "served", "success"] + \
+                                    ["return:" + a for a in self.possible_agents]
+        self.clear_episode_stats()
+        self._flags |= _native.STEP_EPISODE_STATS
 
     # ------------------------------------------------------------------ helpers
     def _call(self, fn, *args):
@@ -422,6 +451,41 @@ class BatchedCookingEnv:
             _native.check(self.lib.cz_layout_ids(self._handle, out.data_ptr(), self.num_envs, self.seed, self.env_offset,
                                                  int(episode), self._stream()))
         return out
+
+    # ------------------------------------------------------------------ episode statistics
+    def _need_stats(self):
+        if self._stats is None:
+            raise _native.NativeError("episode statistics are off: construct the environment with episode_stats=True")
+        return self._stats
+
+    def episode_stats(self):
+        """Per-environment episode statistics (constructor argument episode_stats=True), as views of the device buffers
+        that every step updates (no copy, no synchronisation; ordered like the step's rewards and flags):
+        "return" f64 [N, A] of the running episode, "last_return" f64 [N, A], "last_length" i32 [N], "last_served" u8 [N]
+        (recipes whose root node is marked) and "last_success" u8 [N] (the end_condition_all_dishes condition) of the last
+        finished episode, "finished" i32 [N] episodes finished since the last clear.  The rule is documented with
+        CZ_STEP_EPISODE_STATS in include/cz_b200.h; a reset needs no extra call."""
+        st = self._need_stats()
+        return {k: st[k] for k in ("return", "last_return", "last_length", "last_served", "last_success", "finished")}
+
+    def episode_totals(self, clear=False):
+        """f64 [4 + A] device copy of the sums over every episode finished since the last clear, named by
+        episode_totals_names: episodes, length, served, success, return:player_i.  The vector sharding.reduce_stats sums
+        over ranks.  clear=True zeroes the accumulator on the same stream after the copy."""
+        st = self._need_stats()
+        s = self.stream if self.stream is not None else torch.cuda.current_stream(self.device)
+        with torch.cuda.stream(s):
+            out = st["totals"].clone()
+            if clear:
+                st["totals"].zero_()
+        return out
+
+    def clear_episode_stats(self):
+        """Start a new counting window (cz_stats_clear): returns, the last-episode fields, finished and the totals become
+        0; an episode that has not taken a step yet is counted whole, one already running is not counted."""
+        self._need_stats()
+        with torch.cuda.device(self.device):
+            _native.check(self.lib.cz_stats_clear(self._handle, self.state.data_ptr(), self.num_envs, self._stream()))
 
     # ------------------------------------------------------------------ state import/export
     def export_state(self, env=None):

@@ -1030,6 +1030,7 @@ cz_obs_any_whole_kernel(const __grid_constant__ CzDev T, const uint32_t* __restr
 }
 
 #include "cz_grid.cuh"
+#include "cz_stats.cuh"
 
 // =========================================================================================
 // Host side: tables object and the C ABI
@@ -1087,6 +1088,7 @@ struct cz_tables {
                          // loops over its tiles runs in the background of the row writer instead of displacing it
   size_t smem_optin;
   CzGridDev grid;           // the grid observation writer's constants (cz_grid.cuh)
+  CzStatsDev stats;         // episode statistics buffers of cz_stats_attach (stats.n == 0: none attached)
 };
 
 template <typename Tp>
@@ -1378,8 +1380,12 @@ extern "C" int cz_tables_create(const cz_table_desc* d, int device, cz_tables** 
   SET_SMEM(cz_obs_any_kernel<true>); SET_SMEM(cz_obs_any_kernel<false>); SET_SMEM(cz_obs_any_whole_kernel);
   SET_SMEM((cz_obs_whole_kernel<2, false>)); SET_SMEM((cz_obs_whole_kernel<3, false>)); SET_SMEM((cz_obs_whole_kernel<4, false>));
   SET_SMEM((cz_obs_whole_kernel<2, true>)); SET_SMEM((cz_obs_whole_kernel<3, true>)); SET_SMEM((cz_obs_whole_kernel<4, true>));
-  SET_SMEM((cz_warp_kernel<1, 16>)); SET_SMEM((cz_warp_kernel<2, 16>)); SET_SMEM((cz_warp_kernel<3, 16>)); SET_SMEM((cz_warp_kernel<4, 16>));
-  SET_SMEM((cz_warp_kernel<1, 32>)); SET_SMEM((cz_warp_kernel<2, 32>)); SET_SMEM((cz_warp_kernel<3, 32>)); SET_SMEM((cz_warp_kernel<4, 32>));
+#define SET_WARP(S)                                                                                                     \
+  SET_SMEM((cz_warp_kernel<1, 16, S>)); SET_SMEM((cz_warp_kernel<2, 16, S>)); SET_SMEM((cz_warp_kernel<3, 16, S>));    \
+  SET_SMEM((cz_warp_kernel<4, 16, S>)); SET_SMEM((cz_warp_kernel<1, 32, S>)); SET_SMEM((cz_warp_kernel<2, 32, S>));    \
+  SET_SMEM((cz_warp_kernel<3, 32, S>)); SET_SMEM((cz_warp_kernel<4, 32, S>))
+  SET_WARP(false); SET_WARP(true);
+#undef SET_WARP
 #undef SET_MODE
 #undef SET_SMEM
   *out = t;
@@ -1610,13 +1616,66 @@ extern "C" int cz_random_actions(const cz_tables* t, uint8_t* actions, int n_env
 
 static int cz_pipe_init(cz_tables* t);
 
+// ---- episode statistics (cz_stats.cuh) ------------------------------------------------------------------------------
+extern "C" int cz_stats_attach(cz_tables* t, const cz_stats_desc* d) {
+  if (!t) return cz_fail(CZ_EINVAL, "%s", "null argument");
+  if (!d) {
+    memset(&t->stats, 0, sizeof(t->stats));
+    return CZ_OK;
+  }
+  if (d->n_envs < 1 || !d->ret || !d->episode || !d->open || !d->last_ret || !d->last_len || !d->last_served ||
+      !d->last_success || !d->finished || !d->totals)
+    return cz_fail(CZ_EINVAL, "%s", "cz_stats_attach: every buffer is required and n_envs must be at least 1");
+  CzStatsDev& S = t->stats;
+  S.ret = d->ret; S.episode = d->episode; S.open = d->open; S.last_ret = d->last_ret; S.last_len = d->last_len;
+  S.last_served = d->last_served; S.last_success = d->last_success; S.finished = d->finished; S.totals = d->totals;
+  S.n = d->n_envs;
+  return CZ_OK;
+}
+
+// CZ_STEP_EPISODE_STATS needs attached statistics of exactly this batch
+static int cz_stats_check(const cz_tables* t, int n_envs) {
+  if (t->stats.n == 0) return cz_fail(CZ_EINVAL, "%s", "CZ_STEP_EPISODE_STATS without statistics attached (cz_stats_attach)");
+  if (t->stats.n != n_envs) return cz_fail(CZ_EINVAL, "%s", "CZ_STEP_EPISODE_STATS: n_envs differs from the attached statistics");
+  return CZ_OK;
+}
+
+// the record update after one step of all n_envs environments of `state` (post-step state, reward of that step)
+static int cz_stats_launch(const cz_tables* t, const uint32_t* state, const double* reward, int n_envs, cudaStream_t s) {
+  const CzDev& T = t->dev;
+  const uint32_t* misc = state + (size_t)(T.D + T.A) * n_envs;
+  const int blocks = (n_envs + CZ_STATS_THREADS - 1) / CZ_STATS_THREADS;
+  switch (T.A) {
+    case 1: cz_stats_kernel<1><<<blocks, CZ_STATS_THREADS, 0, s>>>(t->stats, misc, reward, n_envs, n_envs, T.R, T.end_all); break;
+    case 2: cz_stats_kernel<2><<<blocks, CZ_STATS_THREADS, 0, s>>>(t->stats, misc, reward, n_envs, n_envs, T.R, T.end_all); break;
+    case 3: cz_stats_kernel<3><<<blocks, CZ_STATS_THREADS, 0, s>>>(t->stats, misc, reward, n_envs, n_envs, T.R, T.end_all); break;
+    default: cz_stats_kernel<4><<<blocks, CZ_STATS_THREADS, 0, s>>>(t->stats, misc, reward, n_envs, n_envs, T.R, T.end_all); break;
+  }
+  g_launches.fetch_add(1);
+  CZ_CUDA(cudaGetLastError());
+  return CZ_OK;
+}
+
+extern "C" int cz_stats_clear(const cz_tables* t, const uint32_t* state, int n_envs, void* stream) {
+  if (!t || !state) return cz_fail(CZ_EINVAL, "%s", "null argument");
+  int rc = cz_stats_check(t, n_envs);
+  if (rc != CZ_OK) return rc;
+  const CzDev& T = t->dev;
+  const int blocks = (n_envs + CZ_STATS_THREADS - 1) / CZ_STATS_THREADS;
+  cz_stats_clear_kernel<<<blocks, CZ_STATS_THREADS, 0, (cudaStream_t)stream>>>(t->stats, state + (size_t)(T.D + T.A) * n_envs,
+                                                                               n_envs, n_envs, T.A);
+  g_launches.fetch_add(1);
+  CZ_CUDA(cudaGetLastError());
+  return CZ_OK;
+}
+
 // In-place step of a large batch as `split` column ranges: the dynamics of range c + 1 (internal high-priority stream)
 // run under the row writer of range c (second internal stream), so only the first range's dynamics are exposed.  The
 // caller's stream forks into both and joins them again: every output is ordered on it when the call's work is done,
 // exactly like the two launches it replaces.
 static int cz_step_split(cz_tables* t, uint32_t* state, const uint8_t* actions, double* obs, double* reward,
                          uint8_t* terminated, uint8_t* truncated, uint32_t* error_flags, int n_envs, uint32_t flags,
-                         uint64_t seed, int64_t env_offset, void* stream) {
+                         uint64_t seed, int64_t env_offset, void* stream, bool stats) {
   int rc = cz_pipe_init(t);
   if (rc != CZ_OK) return rc;
   const int A = t->dev.A, L = t->dev.L;
@@ -1638,6 +1697,10 @@ static int cz_step_split(cz_tables* t, uint32_t* state, const uint8_t* actions, 
     rc = cz_launch_obs64(t, state + e0, obs + na * L, n, t->pipe_obs, n_envs);
     if (rc != CZ_OK) return rc;
   }
+  if (stats) {  // one launch over all n after every range's dynamics, before the event the caller's stream waits on
+    rc = cz_stats_launch(t, state, reward, n_envs, t->pipe_dyn);
+    if (rc != CZ_OK) return rc;
+  }
   CZ_CUDA(cudaEventRecord(t->ev_dyn, t->pipe_dyn));
   CZ_CUDA(cudaEventRecord(t->ev_obs[0], t->pipe_obs));
   CZ_CUDA(cudaStreamWaitEvent(user, t->ev_dyn, 0));
@@ -1646,16 +1709,18 @@ static int cz_step_split(cz_tables* t, uint32_t* state, const uint8_t* actions, 
 }
 
 // one in-place step with resident actions on the lane-per-environment kernels
-static int cz_step_one(const cz_tables* t, uint32_t* state, const uint8_t* actions, double* obs, double* reward,
-                       uint8_t* terminated, uint8_t* truncated, uint32_t* error_flags, int n_envs, uint32_t flags,
-                       uint64_t seed, int64_t env_offset, void* stream) {
+static int cz_step_kernels(const cz_tables* t, uint32_t* state, const uint8_t* actions, double* obs, double* reward,
+                           uint8_t* terminated, uint8_t* truncated, uint32_t* error_flags, int n_envs, uint32_t flags,
+                           uint64_t seed, int64_t env_offset, void* stream, bool stats, bool* stats_done) {
   // 33-64 pair plans always, and large batches of the other packed plans (the short-block row writer streams faster than the
   // observation phase of the fused kernel; small batches keep the single launch): dynamics, then the row writer
   if (t && obs && !(flags & CZ_STEP_OBS_F32) &&
       (t->simple2 || (t->simple && t->two_kernel_min_envs > 0 && n_envs >= t->two_kernel_min_envs))) {
-    if (t->split > 1 && n_envs >= 2 * t->two_kernel_min_envs && t->two_kernel_min_envs > 0)
+    if (t->split > 1 && n_envs >= 2 * t->two_kernel_min_envs && t->two_kernel_min_envs > 0) {
+      *stats_done = stats;  // the split step updates the statistics on its dynamics stream
       return cz_step_split(const_cast<cz_tables*>(t), state, actions, obs, reward, terminated, truncated, error_flags, n_envs, flags,
-                           seed, env_offset, stream);
+                           seed, env_offset, stream, stats);
+    }
     int rc = cz_launch<MODE_STEP>(t, state, state, true, actions, nullptr, nullptr, nullptr, nullptr, reward, terminated, truncated,
                                   error_flags, n_envs, flags, seed, env_offset, stream);
     if (rc != CZ_OK) return rc;
@@ -1680,10 +1745,22 @@ static int cz_step_one(const cz_tables* t, uint32_t* state, const uint8_t* actio
                               error_flags, n_envs, flags, seed, env_offset, stream);
 }
 
+// one in-place step on the per-step kernels; with `stats`, the record update follows the step's kernels on `stream` (the
+// split step launches it itself, on its dynamics stream)
+static int cz_step_one(const cz_tables* t, uint32_t* state, const uint8_t* actions, double* obs, double* reward,
+                       uint8_t* terminated, uint8_t* truncated, uint32_t* error_flags, int n_envs, uint32_t flags,
+                       uint64_t seed, int64_t env_offset, void* stream, bool stats) {
+  bool stats_done = false;
+  int rc = cz_step_kernels(t, state, actions, obs, reward, terminated, truncated, error_flags, n_envs, flags, seed, env_offset,
+                           stream, stats, &stats_done);
+  if (rc != CZ_OK || !stats || stats_done) return rc;
+  return cz_stats_launch(t, state, reward, n_envs, (cudaStream_t)stream);
+}
+
 // k_steps consecutive steps of every environment in ONE launch of the warp-per-environment kernel
 static int cz_launch_warp(const cz_tables* t, uint32_t* state, const uint8_t* actions, double* obs, double* reward,
                           uint8_t* terminated, uint8_t* truncated, uint32_t* error_flags, int n_envs, int k_steps, uint32_t flags,
-                          uint64_t seed, int64_t env_offset, uint64_t action_step, void* stream) {
+                          uint64_t seed, int64_t env_offset, uint64_t action_step, void* stream, bool stats) {
   if (((uintptr_t)obs & 15) != 0) return cz_fail(CZ_EINVAL, "%s", "obs must be 16-byte aligned");
   const CzDev& T = t->dev;
   // two environments per warp (16-lane groups) when every dynamic slot finds a lane in half a warp
@@ -1692,13 +1769,21 @@ static int cz_launch_warp(const cz_tables* t, uint32_t* state, const uint8_t* ac
   const int blocks = (n_envs + groups - 1) / groups;
   const size_t smem = wk_smem_bytes(T.V, T.A, CZ_WARP_WHOLE ? T.L : T.stage_len, G);
   cudaStream_t s = (cudaStream_t)stream;
-#define CZ_WARP_GO(NA)                                                                                                          \
+#define CZ_WARP_GO_S(NA, S)                                                                                                    \
   if (G == 16)                                                                                                                 \
-    cz_warp_kernel<NA, 16><<<blocks, 32 * WK_WARPS, smem, s>>>(t->dev, state, actions, obs, reward, terminated, truncated,      \
-                                                               error_flags, n_envs, k_steps, flags, seed, env_offset, action_step); \
+    cz_warp_kernel<NA, 16, S><<<blocks, 32 * WK_WARPS, smem, s>>>(t->dev, state, actions, obs, reward, terminated, truncated,   \
+                                                                  error_flags, n_envs, k_steps, flags, seed, env_offset,         \
+                                                                  action_step, t->stats);                                        \
   else                                                                                                                         \
-    cz_warp_kernel<NA, 32><<<blocks, 32 * WK_WARPS, smem, s>>>(t->dev, state, actions, obs, reward, terminated, truncated,      \
-                                                               error_flags, n_envs, k_steps, flags, seed, env_offset, action_step)
+    cz_warp_kernel<NA, 32, S><<<blocks, 32 * WK_WARPS, smem, s>>>(t->dev, state, actions, obs, reward, terminated, truncated,   \
+                                                                  error_flags, n_envs, k_steps, flags, seed, env_offset,         \
+                                                                  action_step, t->stats)
+#define CZ_WARP_GO(NA)          \
+  if (stats) {                  \
+    CZ_WARP_GO_S(NA, true);     \
+  } else {                      \
+    CZ_WARP_GO_S(NA, false);    \
+  }
   switch (T.A) {
     case 1: CZ_WARP_GO(1); break;
     case 2: CZ_WARP_GO(2); break;
@@ -1706,6 +1791,7 @@ static int cz_launch_warp(const cz_tables* t, uint32_t* state, const uint8_t* ac
     default: CZ_WARP_GO(4); break;
   }
 #undef CZ_WARP_GO
+#undef CZ_WARP_GO_S
   g_launches.fetch_add(1);
   CZ_CUDA(cudaGetLastError());
   return CZ_OK;
@@ -1719,12 +1805,18 @@ extern "C" int cz_step(const cz_tables* t, uint32_t* state, const uint8_t* actio
   const bool dev_actions = (flags & CZ_STEP_DEVICE_ACTIONS) != 0;
   if (!actions && !dev_actions) return cz_fail(CZ_EINVAL, "%s", "actions is NULL and CZ_STEP_DEVICE_ACTIONS is not set");
   if (dev_actions) actions = nullptr;
+  const bool stats = (flags & CZ_STEP_EPISODE_STATS) != 0;
+  if (stats) {
+    int rc = cz_stats_check(t, n_envs);
+    if (rc != CZ_OK) return rc;
+    flags &= ~CZ_STEP_EPISODE_STATS;
+  }
   if (n_envs <= 0) return CZ_OK;
   const CzDev& T = t->dev;
   const bool warp_ok = (t->simple || t->simple2) && !(flags & CZ_STEP_OBS_F32);
   if (warp_ok && (k_steps > 1 ? n_envs <= t->warp_k_max_envs : n_envs <= t->warp_max_envs))
     return cz_launch_warp(t, state, actions, obs, reward, terminated, truncated, error_flags, n_envs, k_steps, flags, seed,
-                          env_offset, action_step, stream);
+                          env_offset, action_step, stream, stats);
   // everything else (generic tables, float32 rows, large batches): k_steps launches of the per-step kernels
   cz_tables* tm = const_cast<cz_tables*>(t);
   if (dev_actions && n_envs > t->rand_envs) {
@@ -1759,7 +1851,7 @@ extern "C" int cz_step(const cz_tables* t, uint32_t* state, const uint8_t* actio
       obs_k = reinterpret_cast<double*>(tm->d_keep);
     }
     int rc = cz_step_one(t, state, a, obs_k, reward + o * na, terminated + o * na, truncated + o * na, error_flags, n_envs,
-                         flags & ~(CZ_STEP_DEVICE_ACTIONS | CZ_STEP_KEEP_ALL), seed, env_offset, stream);
+                         flags & ~(CZ_STEP_DEVICE_ACTIONS | CZ_STEP_KEEP_ALL), seed, env_offset, stream, stats);
     if (rc != CZ_OK) return rc;
     if (dst != obs_k) CZ_CUDA(cudaMemcpyAsync(dst, obs_k, obs_bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   }
@@ -1852,6 +1944,12 @@ extern "C" int cz_step_pipelined(cz_tables* t, uint32_t* state2, const uint8_t* 
                                  uint64_t seed, int64_t env_offset, void* stream) {
   if (!t || !state2 || !actions || !obs || !reward || !terminated || !truncated) return cz_fail(CZ_EINVAL, "%s", "null argument");
   if (!t->simple && !t->simple2) return cz_fail(CZ_EINVAL, "%s", "the pipelined step needs the specialised kernels (see DESIGN.md)");
+  const bool stats = (flags & CZ_STEP_EPISODE_STATS) != 0;
+  if (stats) {
+    int rc = cz_stats_check(t, n_envs);
+    if (rc != CZ_OK) return rc;
+    flags &= ~CZ_STEP_EPISODE_STATS;
+  }
   int rc = cz_pipe_init(t);
   if (rc != CZ_OK) return rc;
   const size_t half = (size_t)t->dev.rows * n_envs;
@@ -1868,6 +1966,10 @@ extern "C" int cz_step_pipelined(cz_tables* t, uint32_t* state2, const uint8_t* 
                             error_flags, n_envs, flags, seed, env_offset, t->pipe_dyn, 0,
                             t->pipe_steps == 0 ? 0 : t->pipe_dyn_blocks);  // nothing to hide behind on the first step: full grid
   if (rc != CZ_OK) return rc;
+  if (stats) {  // on the dynamics stream, before the event that orders the caller's stream: ordered like rewards and flags
+    rc = cz_stats_launch(t, out, reward, n_envs, t->pipe_dyn);
+    if (rc != CZ_OK) return rc;
+  }
   CZ_CUDA(cudaEventRecord(t->ev_dyn, t->pipe_dyn));
   CZ_CUDA(cudaStreamWaitEvent(t->pipe_obs, t->ev_dyn, 0));
   CZ_CUDA(cudaStreamWaitEvent(t->pipe_obs, t->ev_user, 0));
@@ -1912,6 +2014,10 @@ extern "C" int cz_step_host(cz_tables* t, uint32_t* state_dev, const uint8_t* ac
   if (!t || !actions_host || !obs_host || !reward_host || !terminated_host || !truncated_host)
     return cz_fail(CZ_EINVAL, "%s", "null argument");
   const CzDev& T = t->dev;
+  if (flags & CZ_STEP_EPISODE_STATS) {
+    int rc = cz_stats_check(t, n_envs);
+    if (rc != CZ_OK) return rc;
+  }
   if (n_envs > t->scratch_envs) {
     if (t->d_actions) { cudaFree(t->d_actions); cudaFree(t->d_obs); cudaFree(t->d_reward); cudaFree(t->d_term); cudaFree(t->d_trunc); }
     t->scratch_envs = 0;
@@ -1934,6 +2040,8 @@ extern "C" int cz_step_host(cz_tables* t, uint32_t* state_dev, const uint8_t* ac
   if (chunks > 1 && (t->simple || t->simple2) && !(flags & CZ_STEP_OBS_F32) && n_envs >= 4 * 8192) {
     int rc = cz_pipe_init(t);
     if (rc != CZ_OK) return rc;
+    const bool stats = (flags & CZ_STEP_EPISODE_STATS) != 0;
+    flags &= ~CZ_STEP_EPISODE_STATS;
     const int chunk = (((n_envs + chunks - 1) / chunks) + 255) & ~255;
     cudaStream_t copy = t->pipe_obs;
     int c = 0;
@@ -1952,6 +2060,10 @@ extern "C" int cz_step_host(cz_tables* t, uint32_t* state_dev, const uint8_t* ac
       CZ_CUDA(cudaMemcpyAsync(reward_host + o, t->d_reward + o, (size_t)n * T.A * sizeof(double), cudaMemcpyDeviceToHost, copy));
       CZ_CUDA(cudaMemcpyAsync(terminated_host + o, t->d_term + o, (size_t)n * T.A, cudaMemcpyDeviceToHost, copy));
       CZ_CUDA(cudaMemcpyAsync(truncated_host + o, t->d_trunc + o, (size_t)n * T.A, cudaMemcpyDeviceToHost, copy));
+    }
+    if (stats) {  // after every range's step; the copies do not wait for it
+      rc = cz_stats_launch(t, state_dev, t->d_reward, n_envs, s);
+      if (rc != CZ_OK) return rc;
     }
     CZ_CUDA(cudaEventRecord(t->ev_obs[0], copy));
     CZ_CUDA(cudaStreamWaitEvent(s, t->ev_obs[0], 0));

@@ -705,12 +705,20 @@ __host__ __device__ inline size_t wk_smem_bytes(int V, int A, int stage_len, int
   return cz_block_smem_head(V) + 64 * 4 + (size_t)groups * (WK_WORDS * 4 + (size_t)A * ((stage_len + 1) / 2) * 16);
 }
 
-template <int NA, int G>
-__global__ void __launch_bounds__(32 * WK_WARPS, G == 32 ? 7 : 4)
+// STATS (CZ_STEP_EPISODE_STATS): the episode-statistics record of the group's environment (cz_stats.cuh) is loaded in the
+// prologue, updated by cz_stats_rule after every step and written in the epilogue next to the state; lane g < NA holds
+// agent g's running return, and K steps stay one launch.  STATS = false compiles to the kernel without any of it (the same
+// SASS as a kernel without the statistics code); the true instantiation has its own bound for 32-lane groups, where the plain
+// kernel's 7 blocks per SM (72 registers) spill the record.
+#ifndef CZ_WARP_STATS_MIN_BLOCKS32
+#define CZ_WARP_STATS_MIN_BLOCKS32 6
+#endif
+template <int NA, int G, bool STATS>
+__global__ void __launch_bounds__(32 * WK_WARPS, G == 32 ? (STATS ? CZ_WARP_STATS_MIN_BLOCKS32 : 7) : 4)
 cz_warp_kernel(const __grid_constant__ CzDev T, uint32_t* __restrict__ state, const uint8_t* __restrict__ actions,
                double* __restrict__ obs, double* __restrict__ reward, uint8_t* __restrict__ term, uint8_t* __restrict__ trunc,
                uint32_t* __restrict__ errflags, int n_envs, int k_steps, uint32_t flags, uint64_t seed, int64_t env_offset,
-               uint64_t action_step) {
+               uint64_t action_step, const __grid_constant__ CzStatsDev S) {
   constexpr bool FAST = true;
   constexpr int GROUPS = WK_WARPS * 32 / G;  // environments per block
   constexpr int TK = 64 / G;                 // table elements (double2) of a row per lane, at most
@@ -779,6 +787,16 @@ cz_warp_kernel(const __grid_constant__ CzDev T, uint32_t* __restrict__ state, co
   }
   wk_recipe_consts(T, e);
   wk_variant_consts(T, e);
+  // episode statistics: the record, and what the finished episodes of this launch add to it (group-uniform except the
+  // returns, which lane g < NA holds for agent g)
+  uint32_t st_seen = 0, st_open = 0, st_n = 0, st_len = 0, st_served = 0, st_succ = 0;
+  uint32_t st_last = 0;  // the last finished episode: t | served << 20 | success << 28
+  double st_ret[1] = {0.0}, st_sum = 0.0, st_lret = 0.0;
+  if constexpr (STATS) {
+    st_seen = S.episode[env];
+    st_open = S.open[env];
+    if (g < NA) st_ret[0] = S.ret[(size_t)env * NA + g];
+  }
 
   // where this lane's table elements (double2 units g, g + G, ...) land in a row: segment 0 first, then segment 1
   int tdst[TK];
@@ -830,6 +848,22 @@ cz_warp_kernel(const __grid_constant__ CzDev T, uint32_t* __restrict__ state, co
       wk_variant_consts(T, e);
     }
     wk_step_env(T, e, act, fresh, rw, term_mask, trunc_mask, seed, genv);
+    if constexpr (STATS) {
+      double r_mine[1] = {rw[0]};
+#pragma unroll
+      for (int i = 1; i < NA; ++i)
+        if (g == i) r_mine[0] = rw[i];
+      uint32_t served = 0, success = 0;
+      if (cz_stats_rule<1>(st_seen, st_open, st_ret, r_mine, e.episode, e.tinfo, e.marks, T.R, T.end_all != 0, served, success)) {
+        st_n += 1;
+        st_len += TI_T(e.tinfo);
+        st_served += served;
+        st_succ += success;
+        st_last = TI_T(e.tinfo) | served << 20 | success << 28;  // t < 2^20
+        st_sum += st_ret[0];
+        st_lret = st_ret[0];
+      }
+    }
     if (g < NA) {
       double r = rw[0];
 #pragma unroll
@@ -921,4 +955,27 @@ cz_warp_kernel(const __grid_constant__ CzDev T, uint32_t* __restrict__ state, co
     state[(size_t)(D + g) * N + env] = w;
   }
   if (errflags && e.err && g == 0) errflags[env] |= e.err;
+  if constexpr (STATS) {
+    if (g < NA) S.ret[(size_t)env * NA + g] = st_ret[0];
+    if (g == 0) {
+      S.episode[env] = st_seen;
+      S.open[env] = (uint8_t)st_open;
+    }
+    if (st_n) {  // at most one atomicAdd per field and environment per launch, whatever K is
+      if (g < NA) {
+        S.last_ret[(size_t)env * NA + g] = st_lret;
+        atomicAdd(S.totals + 4 + g, st_sum);
+      }
+      if (g == 0) {
+        S.last_len[env] = (int32_t)(st_last & 0xFFFFFu);
+        S.last_served[env] = (uint8_t)((st_last >> 20) & 255u);
+        S.last_success[env] = (uint8_t)(st_last >> 28);
+        S.finished[env] += (int32_t)st_n;
+        atomicAdd(S.totals + 0, (double)st_n);
+        atomicAdd(S.totals + 1, (double)st_len);
+        if (st_served) atomicAdd(S.totals + 2, (double)st_served);
+        if (st_succ) atomicAdd(S.totals + 3, (double)st_succ);
+      }
+    }
+  }
 }

@@ -135,6 +135,39 @@ class MixedAgentCookingEnv:
         self._fan_out(go)
         return self.actions, crashed
 
+    def episode_stats(self):
+        """episode_stats() of every group gathered into population-indexed tensors: [N, A_max] returns (padded agents
+        read 0) and [N] per-environment fields.  Copies, on the caller's stream."""
+        N, A = self.num_envs, self.max_agents
+        out = None
+        for a, g in self.groups.items():
+            st = g.episode_stats()
+            if out is None:
+                out = {k: torch.zeros((N, A) if v.dim() == 2 else (N,), dtype=v.dtype, device=self.device)
+                       for k, v in st.items()}
+            idx = self.index[a]
+            for k, v in st.items():
+                if v.dim() == 2:
+                    out[k][idx, :a] = v
+                else:
+                    out[k][idx] = v
+        return out
+
+    def episode_totals(self, clear=False):
+        """f64 [4 + A_max]: the groups' episode_totals() summed, each padded to A_max return columns"""
+        tot = torch.zeros(4 + self.max_agents, dtype=torch.float64, device=self.device)
+        for a, g in self.groups.items():
+            tot[:4 + a] += g.episode_totals(clear=clear)
+        return tot
+
+    def clear_episode_stats(self):
+        for g in self.groups.values():
+            g.clear_episode_stats()
+
+    @property
+    def episode_totals_names(self):
+        return ["episodes", "length", "served", "success"] + ["return:player_" + str(i) for i in range(self.max_agents)]
+
     def close(self):
         for g in self.groups.values():
             g.close()

@@ -91,6 +91,38 @@ extern "C" {
                                   counter stream of cz_random_actions at step index action_step + k */
 #define CZ_STEP_KEEP_ALL 8u    /* cz_step with k_steps > 1: obs / reward / terminated / truncated are [k_steps][...] arrays and
                                   every step's outputs are kept; without it each step overwrites the same [n][A][...] buffers */
+#define CZ_STEP_EPISODE_STATS 16u /* update the episode statistics attached with cz_stats_attach after every step of every
+                                  environment (honoured by cz_step, cz_step_pipelined and cz_step_host; CZ_EINVAL when no
+                                  statistics are attached or their n_envs differs from the call's) */
+
+/* ---- episode statistics ----------------------------------------------------------------------
+ * Every environment carries a record (cz_stats_desc).  After each step of the environment, with the post-step rows EPISODE,
+ * TINFO (t, done) and MARKS and that step's rewards r[a]:
+ *   1. EPISODE != episode: a reset happened since the last step (cz_reset, masked or not, or an auto-reset step):
+ *      episode = EPISODE, ret[:] = 0, open = 1.
+ *   2. open: ret[a] = ret[a] + r[a] for every agent (float64, round to nearest, in step order).
+ *   3. open and TINFO's done bit: the episode just finished.  last_ret = ret, last_len = t, last_served = number of the R
+ *      recipes whose root mark (bit 0 of MARKS byte r) is set, last_success = the recipe condition of
+ *      end_condition_all_dishes (all R recipes if set, any if not; a time-up alone gives 0), finished += 1,
+ *      totals += (1, t, served, success, ret[0..A)), open = 0.
+ * An auto-reset step has reward 0 and leaves t = 0, so it adds nothing; without auto-reset a finished environment that keeps
+ * stepping is counted once.  The record keeps only the LAST finished episode: when one call of K steps can finish several
+ * episodes of an environment, read the totals.
+ * totals f64 [4 + A]: episodes, sum of lengths, recipes served, successes, then the return sum of each agent.  The first four
+ * are integers held exactly; the return sums are added per block and then across blocks with atomics, so their last bits
+ * depend on the summation order (run to run they may differ by rounding; the per-environment fields never do). */
+typedef struct cz_stats_desc {
+  int32_t n_envs;
+  double* ret;             /* [n][A] return of the running episode                                   */
+  uint32_t* episode;       /* [n] internal: EPISODE row the record has seen last                     */
+  uint8_t* open;           /* [n] internal: the running episode is being counted                     */
+  double* last_ret;        /* [n][A] return of the last finished episode                             */
+  int32_t* last_len;       /* [n] its length (t at done)                                             */
+  uint8_t* last_served;    /* [n] its recipes served                                                 */
+  uint8_t* last_success;   /* [n] its recipe condition (0 / 1)                                       */
+  int32_t* finished;       /* [n] episodes finished since cz_stats_clear                             */
+  double* totals;          /* [4 + A] sums since cz_stats_clear (layout above)                       */
+} cz_stats_desc;
 
 /* Host-side description of everything compiled once per (level, meta, recipes, scheme):
  * replaces load_level.load_level / parsing.parse_* (engine/load_level.py:55-71,
@@ -186,6 +218,14 @@ int cz_layout_ids(const cz_tables* t, int32_t* layout_ids, int n_envs, uint64_t 
 int cz_step(const cz_tables* t, uint32_t* state, const uint8_t* actions, double* obs, double* reward,
             uint8_t* terminated, uint8_t* truncated, uint32_t* error_flags, int n_envs, int k_steps,
             uint32_t flags, uint64_t seed, int64_t env_offset, uint64_t action_step, void* stream);
+
+/* Attach caller-owned device buffers for CZ_STEP_EPISODE_STATS (NULL detaches).  Every pointer is required and n_envs >= 1,
+ * or CZ_EINVAL.  The tables keep the pointers, not the buffers: they must outlive the attachment. */
+int cz_stats_attach(cz_tables* t, const cz_stats_desc* desc);
+/* Start a counting window (one small kernel on `stream`): ret, the last_* fields, finished and the totals become 0,
+ * episode = EPISODE and open = (t == 0), so an episode that has not taken a step yet is counted whole and one already
+ * running is not counted at all. */
+int cz_stats_clear(const cz_tables* t, const uint32_t* state, int n_envs, void* stream);
 
 /* get_feature_vector only (cooking_env.py:352-373): rebuild obs from the current state. */
 int cz_observe(const cz_tables* t, const uint32_t* state, double* obs, int n_envs, void* stream);
