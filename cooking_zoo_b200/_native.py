@@ -17,6 +17,7 @@ STEP_OBS_F32 = 2
 STEP_DEVICE_ACTIONS = 4
 STEP_KEEP_ALL = 8
 STEP_EPISODE_STATS = 16
+STEP_COOK_AGENTS = 32
 ERR_BITS = {1: "CUTBOARD_NONE", 2: "REMOVE", 4: "SWITCH_LINK", 8: "SPAWN_LOC", 16: "TRUNC_DESPAWN", 32: "OBS_OVERFLOW",
             64: "OFFGRID", 128: "BAD_ID"}
 
@@ -50,6 +51,11 @@ class StatsDesc(C.Structure):
                                                             "last_success", "finished", "totals")]
 
 
+class CookDesc(C.Structure):
+    _fields_ = [("n_envs", C.c_int32), ("k_capacity", C.c_int32)] + \
+               [(n, _P) for n in ("agent_mask", "cook_recipes", "actions_taken", "crashed")]
+
+
 # every symbol include/cz_b200.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "cz_abi_version": (C.c_int, []),
@@ -81,6 +87,7 @@ SIGNATURES = {
     "cz_policy_destroy": (C.c_int, [_P]),
     "cz_policy_config": (C.c_int, [_P, C.c_int]),
     "cz_policy_act": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, _P]),
+    "cz_cook_attach": (C.c_int, [_P, _P, C.POINTER(CookDesc)]),
     "cz_random_actions": (C.c_int, [_P, _P, C.c_int, C.c_uint64, C.c_uint64, C.c_int64, _P]),
     "cz_step_host": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int, C.c_uint32, C.c_uint64, C.c_int64, _P]),
 }

@@ -46,7 +46,8 @@ class BatchedCookingEnv:
                  reward_scheme=None, agent_respawn_rate=0.0, grace_period=20, agent_despawn_rate=0.0, *,
                  device="cuda:0", recipe_pool=None, layout_pool_size="auto", layout_seed=0, layouts=None,
                  auto_reset=False, seed=0, env_offset=0, pipelined=False, obs_dtype=torch.float64, stream=None,
-                 pipeline_buffers=2, background_dynamics=0, background_policy=0, episode_stats=False):
+                 pipeline_buffers=2, background_dynamics=0, background_policy=0, episode_stats=False, cook_agents=None,
+                 cook_recipes=None):
         obs_spaces = obs_spaces or ["feature_vector"] * num_agents
         if obs_spaces and all(o == "grid" for o in obs_spaces):
             # per-cell u8 planes [N, A, C, H, W] written by their own kernel after the dynamics (cooking_zoo_b200.grid)
@@ -123,6 +124,78 @@ class BatchedCookingEnv:
         self._stats = None
         if episode_stats:
             self._attach_episode_stats()
+        self._cook = None
+        if cook_agents is not None:
+            self._attach_cook(cook_agents, cook_recipes)
+        elif cook_recipes is not None:
+            raise ValueError("cook_recipes applies to the agents named by cook_agents")
+
+    def _attach_cook(self, cook_agents, cook_recipes):
+        """agents driven by the device cook inside every step (CZ_STEP_COOK_AGENTS, cz_cook_attach)"""
+        N, A, dev = self.num_envs, self.num_agents, self.device
+        mask = self._cook_mask(cook_agents)
+        rid = self._cook_recipe_ids(cook_recipes) if cook_recipes is not None else None
+        policy = self._policy_handle()
+        self._cook = {"mask": mask, "recipes": rid, "policy": policy,
+                      "taken": torch.zeros((N, A), dtype=torch.uint8, device=dev), "bound": None}
+        self.cook_step_crashed = torch.zeros((N,), dtype=torch.uint8, device=dev)
+        self._cook_use(self._cook["taken"], 1)
+        self._flags |= _native.STEP_COOK_AGENTS
+
+    def _cook_use(self, taken, k_capacity, crashed=None):
+        """attach `taken` ([k_capacity, N, A] or [N, A]) as actions_taken of the next calls; host bookkeeping only"""
+        ck = self._cook
+        crashed = self.cook_step_crashed if crashed is None else crashed
+        key = (taken.data_ptr(), int(k_capacity), crashed.data_ptr())
+        if ck["bound"] != key:
+            d = _native.CookDesc()
+            d.n_envs, d.k_capacity = self.num_envs, int(k_capacity)
+            d.agent_mask, d.actions_taken, d.crashed = ck["mask"].data_ptr(), taken.data_ptr(), crashed.data_ptr()
+            d.cook_recipes = ck["recipes"].data_ptr() if ck["recipes"] is not None else None
+            _native.check(self.lib.cz_cook_attach(self._handle, ck["policy"], C.byref(d)))
+            ck["bound"] = key
+        self.actions_taken = taken
+
+    def _cook_mask(self, agents):
+        """cook_agents (agent indices, the same in every environment, or a bool tensor [N, A]) -> u8 bit mask [N] on the
+        device"""
+        N, A = self.num_envs, self.num_agents
+        if isinstance(agents, torch.Tensor):
+            if agents.dtype != torch.bool or tuple(agents.shape) != (N, A):
+                raise ValueError("cook_agents must be a list of agent indices or a bool tensor [num_envs, num_agents]")
+            bits = torch.tensor([1 << i for i in range(A)], dtype=torch.int32, device=self.device)
+            return (agents.to(self.device).to(torch.int32) * bits).sum(1).to(torch.uint8).contiguous()
+        idx = [int(i) for i in agents]
+        if any(i < 0 or i >= A for i in idx):
+            raise ValueError(f"cook_agents: agent indices must lie in 0..{A - 1}")
+        m = 0
+        for i in idx:
+            m |= 1 << i
+        return torch.full((N,), m, dtype=torch.uint8, device=self.device)
+
+    def _cook_recipe_ids(self, cook_recipes):
+        """a list of A recipe names or a [N, A] tensor of indices into tables.recipe_names -> u8 [N, A] on the device"""
+        N, A = self.num_envs, self.num_agents
+        if not isinstance(cook_recipes, torch.Tensor):
+            names = list(cook_recipes)
+            if len(names) != A or any(n not in self.tables.recipe_names for n in names):
+                raise ValueError("cook_recipes must name one recipe of tables.recipe_names per agent "
+                                 "(pass the names in recipe_pool)")
+            cook_recipes = torch.tensor([self.tables.recipe_names.index(n) for n in names],
+                                        dtype=torch.uint8).expand(N, A)
+        rid = cook_recipes.to(device=self.device, dtype=torch.uint8).contiguous()
+        if rid.shape != (N, A):
+            raise ValueError("cook_recipes must have shape [num_envs, num_agents]")
+        return rid
+
+    def set_cook_agents(self, agents):
+        """Change which agents the device cook drives (same forms as the constructor's cook_agents), e.g. between
+        episodes: the mask buffer is rewritten on this environment's stream, so calls enqueued after this one see it."""
+        if self._cook is None:
+            raise _native.NativeError("cook agents are off: construct the environment with cook_agents=...")
+        s = self.stream if self.stream is not None else torch.cuda.current_stream(self.device)
+        with torch.cuda.stream(s):
+            self._cook["mask"].copy_(self._cook_mask(agents))
 
     def _attach_episode_stats(self):
         """episode statistics on the device (cz_stats_attach): every step path updates them from here on"""
@@ -246,6 +319,8 @@ class BatchedCookingEnv:
             # (cz_step_pipelined orders it), so the buffer is never overwritten while a dynamics kernel still reads it
             self._actions.copy_(a)
             a = self._actions
+        if self._cook is not None:
+            self._cook_use(self._cook["taken"], 1)
         if self.pipelined:
             return self._step_pipelined(a)
         self._call(self.lib.cz_step, self._handle, self.state.data_ptr(), a.data_ptr(), self.obs.data_ptr(),
@@ -260,7 +335,10 @@ class BatchedCookingEnv:
         actions: uint8 [k_steps, N, A] on the device, or None: step j's actions are drawn on the device from the
         counter stream of random_actions() at step index action_step + j.  keep_all=False: the usual output buffers
         hold the LAST step's observations / rewards / flags.  keep_all=True: returns fresh [k_steps, ...] tensors with
-        every step's outputs.  Not available in pipelined mode."""
+        every step's outputs.  Not available in pipelined mode.
+
+        With cook_agents, the cook decides for its agents before every step (their columns of `actions` are ignored)
+        and actions_taken holds the applied actions: [N, A] of the last step, or a fresh [k_steps, N, A] with keep_all."""
         if self.pipelined:
             raise _native.NativeError("step_k runs on the in-place state (pipelined=False)")
         N, A, L, K = self.num_envs, self.num_agents, self.obs_len, int(k_steps)
@@ -275,6 +353,11 @@ class BatchedCookingEnv:
             a = a.to(device=self.device, dtype=torch.uint8).contiguous()
             self._k_actions = a          # keep alive until the launch has consumed it
             a_ptr = a.data_ptr()
+        if self._cook is not None:
+            if keep_all:
+                self._cook_use(torch.empty((K, N, A), dtype=torch.uint8, device=self.device), K)
+            else:
+                self._cook_use(self._cook["taken"], 1)
         if keep_all:
             flags |= _native.STEP_KEEP_ALL
             obs = torch.empty((K, N, A, L), dtype=self.obs_dtype, device=self.device)
@@ -298,6 +381,8 @@ class BatchedCookingEnv:
         if a.dtype != torch.uint8 or a.device != self.device or not a.is_contiguous():
             self._actions.copy_(a)
             a = self._actions
+        if self._cook is not None:
+            self._cook_use(self._cook["taken"], 1)
         s = self._stream()
         self._call(self.lib.cz_step, self._handle, self.state.data_ptr(), a.data_ptr(), None, self.reward.data_ptr(),
                    self.terminated.data_ptr(), self.truncated.data_ptr(), self.error_flags.data_ptr(), self.num_envs, 1,
@@ -319,6 +404,9 @@ class BatchedCookingEnv:
             a = a.to(device=self.device, dtype=torch.uint8).contiguous()
             self._k_actions = a          # keep alive until the launch has consumed it
         s = self._stream()
+        cook = self._cook is not None
+        if cook:
+            self._cook_use(self._cook["taken"], 1)
         with torch.cuda.device(self.device):
             if not keep_all:
                 _native.check(self.lib.cz_step(self._handle, self.state.data_ptr(), None if actions is None else a.data_ptr(),
@@ -331,12 +419,23 @@ class BatchedCookingEnv:
             rew = torch.empty((K, N, A), dtype=torch.float64, device=self.device)
             term = torch.empty((K, N, A), dtype=torch.uint8, device=self.device)
             trunc = torch.empty((K, N, A), dtype=torch.uint8, device=self.device)
+            if cook:   # slice j of the applied actions per single step; the raise bits ORed over the K steps
+                taken = torch.empty((K, N, A), dtype=torch.uint8, device=self.device)
+                crash_j = torch.empty_like(self.cook_step_crashed)
             for j in range(K):
+                if cook:
+                    self._cook_use(taken[j], 1, None if j == 0 else crash_j)
                 _native.check(self.lib.cz_step(self._handle, self.state.data_ptr(),
                                                None if actions is None else a[j].data_ptr(), None, rew[j].data_ptr(),
                                                term[j].data_ptr(), trunc[j].data_ptr(), self.error_flags.data_ptr(), N, 1,
                                                flags, self.seed, self.env_offset, int(action_step) + j, s))
                 _native.check(self.lib.cz_observe_grid(self._handle, self.state.data_ptr(), obs[j].data_ptr(), N, s))
+                if cook and j > 0:
+                    with torch.cuda.stream(self.stream if self.stream is not None else torch.cuda.current_stream(self.device)):
+                        self.cook_step_crashed |= crash_j
+            if cook:   # the tables keep the env's own buffers attached, not the temporaries of this call
+                self._cook_use(self._cook["taken"], 1)
+                self.actions_taken = taken
         return obs, rew, term, trunc, self._info
 
     def _observe_grid(self):
@@ -391,29 +490,12 @@ class BatchedCookingEnv:
         cook_recipes: None (cook i follows recipe i of its environment), a list of A recipe names, or a
         uint8 tensor [N, A] of indices into tables.recipe_names.  Returns (actions u8 [N, A], crashed u8 [N]):
         bit i of crashed[e] is set where the reference cook would raise (its action is 0)."""
-        from .policy import compile_policy_tables
         N, A = self.num_envs, self.num_agents
-        if getattr(self, "_policy", None) is None:
-            desc, self._policy_keep = _native.make_policy_desc(self.tables, compile_policy_tables(self.tables))
-            handle = C.c_void_p()
-            _native.check(self.lib.cz_policy_create(self._handle, C.byref(desc), C.byref(handle)))
-            self._policy = handle
-            if self.background_policy:
-                _native.check(self.lib.cz_policy_config(handle, self.background_policy))
+        self._policy_handle()
+        if getattr(self, "cook_actions", None) is None:
             self.cook_actions = torch.zeros((N, A), dtype=torch.uint8, device=self.device)
             self.cook_crashed = torch.zeros((N,), dtype=torch.uint8, device=self.device)
-        rid = None
-        if cook_recipes is not None:
-            if not isinstance(cook_recipes, torch.Tensor):
-                names = list(cook_recipes)
-                if len(names) != A or any(n not in self.tables.recipe_names for n in names):
-                    raise ValueError("cook_recipes must name one recipe of tables.recipe_names per agent "
-                                     "(pass the names in recipe_pool)")
-                cook_recipes = torch.tensor([self.tables.recipe_names.index(n) for n in names],
-                                            dtype=torch.uint8).expand(N, A)
-            rid = cook_recipes.to(device=self.device, dtype=torch.uint8).contiguous()
-            if rid.shape != (N, A):
-                raise ValueError("cook_recipes must have shape [num_envs, num_agents]")
+        rid = self._cook_recipe_ids(cook_recipes) if cook_recipes is not None else None
         with torch.cuda.device(self.device):
             if self.pipelined:     # the cook reads the state only: the observation rows may still be streaming out
                 _native.check(self.lib.cz_pipeline_wait_state(self._handle, self._stream()))
@@ -422,6 +504,18 @@ class BatchedCookingEnv:
                                                  self.cook_actions.data_ptr(), self.cook_crashed.data_ptr(), N,
                                                  self._stream()))
         return self.cook_actions, self.cook_crashed
+
+    def _policy_handle(self):
+        """the device cook's policy (cz_policy_create), created on first use and shared by heuristic_actions and cook_agents"""
+        if getattr(self, "_policy", None) is None:
+            from .policy import compile_policy_tables
+            desc, self._policy_keep = _native.make_policy_desc(self.tables, compile_policy_tables(self.tables))
+            handle = C.c_void_p()
+            _native.check(self.lib.cz_policy_create(self._handle, C.byref(desc), C.byref(handle)))
+            self._policy = handle
+            if self.background_policy:
+                _native.check(self.lib.cz_policy_config(handle, self.background_policy))
+        return self._policy
 
     def observe(self):
         with torch.cuda.device(self.device):

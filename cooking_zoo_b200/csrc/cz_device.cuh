@@ -440,12 +440,13 @@ __device__ __forceinline__ void cz_refresh_plate_free(const CzDev& T, EnvRegs& e
 // the `for obj in world.world_objects[node.name]` loop of Recipe.update_recipe_state
 // (recipe.py:83-87) with check_conditions' attribute test (:96-98).  Out of line: it is called
 // for every node of every recipe and would otherwise be replicated by the unrolled caller.
+template <int S = OSTRIDE>  // S: words between slot records (1: the warp kernel's cook scratch, cz_policy_dev.cuh)
 __device__ __noinline__ uint64_t cz_node_mask(const uint32_t* o, uint32_t span) {
   const uint32_t need = span >> 16;  // O_PRESENT plus the chopped / mashed bit the node asks for
   const int base = span & 255u, end = base + ((span >> 8) & 255u);  // no slots: a type the meta file does not know
   uint64_t mask = 0;
   for (int s = base; s < end; ++s) {
-    uint32_t r = o[s * OSTRIDE];
+    uint32_t r = o[s * S];
     if ((r & need) == need) mask |= 1ull << O_XY(r);
   }
   return mask;

@@ -1031,6 +1031,7 @@ cz_obs_any_whole_kernel(const __grid_constant__ CzDev T, const uint32_t* __restr
 
 #include "cz_grid.cuh"
 #include "cz_stats.cuh"
+#include "cz_policy_dev.cuh"
 
 // =========================================================================================
 // Host side: tables object and the C ABI
@@ -1089,6 +1090,7 @@ struct cz_tables {
   size_t smem_optin;
   CzGridDev grid;           // the grid observation writer's constants (cz_grid.cuh)
   CzStatsDev stats;         // episode statistics buffers of cz_stats_attach (stats.n == 0: none attached)
+  CzCookDev cook;           // CZ_STEP_COOK_AGENTS buffers and policy of cz_cook_attach (cook.n == 0: none attached)
 };
 
 template <typename Tp>
@@ -1380,11 +1382,11 @@ extern "C" int cz_tables_create(const cz_table_desc* d, int device, cz_tables** 
   SET_SMEM(cz_obs_any_kernel<true>); SET_SMEM(cz_obs_any_kernel<false>); SET_SMEM(cz_obs_any_whole_kernel);
   SET_SMEM((cz_obs_whole_kernel<2, false>)); SET_SMEM((cz_obs_whole_kernel<3, false>)); SET_SMEM((cz_obs_whole_kernel<4, false>));
   SET_SMEM((cz_obs_whole_kernel<2, true>)); SET_SMEM((cz_obs_whole_kernel<3, true>)); SET_SMEM((cz_obs_whole_kernel<4, true>));
-#define SET_WARP(S)                                                                                                     \
-  SET_SMEM((cz_warp_kernel<1, 16, S>)); SET_SMEM((cz_warp_kernel<2, 16, S>)); SET_SMEM((cz_warp_kernel<3, 16, S>));    \
-  SET_SMEM((cz_warp_kernel<4, 16, S>)); SET_SMEM((cz_warp_kernel<1, 32, S>)); SET_SMEM((cz_warp_kernel<2, 32, S>));    \
-  SET_SMEM((cz_warp_kernel<3, 32, S>)); SET_SMEM((cz_warp_kernel<4, 32, S>))
-  SET_WARP(false); SET_WARP(true);
+#define SET_WARP(C, S)                                                                                                        \
+  SET_SMEM((cz_warp_kernel<1, 16, C, S>)); SET_SMEM((cz_warp_kernel<2, 16, C, S>)); SET_SMEM((cz_warp_kernel<3, 16, C, S>));    \
+  SET_SMEM((cz_warp_kernel<4, 16, C, S>)); SET_SMEM((cz_warp_kernel<1, 32, C, S>)); SET_SMEM((cz_warp_kernel<2, 32, C, S>));    \
+  SET_SMEM((cz_warp_kernel<3, 32, C, S>)); SET_SMEM((cz_warp_kernel<4, 32, C, S>))
+  SET_WARP(false, false); SET_WARP(false, true); SET_WARP(true, false); SET_WARP(true, true);
 #undef SET_WARP
 #undef SET_MODE
 #undef SET_SMEM
@@ -1669,6 +1671,17 @@ extern "C" int cz_stats_clear(const cz_tables* t, const uint32_t* state, int n_e
   return CZ_OK;
 }
 
+// CZ_STEP_COOK_AGENTS needs attached buffers of exactly this batch, with room for every step a KEEP_ALL call keeps
+static int cz_cook_check(const cz_tables* t, int n_envs, int k_steps, uint32_t flags) {
+  if (t->cook.n == 0) return cz_fail(CZ_EINVAL, "%s", "CZ_STEP_COOK_AGENTS without buffers attached (cz_cook_attach)");
+  if (t->cook.n != n_envs) return cz_fail(CZ_EINVAL, "%s", "CZ_STEP_COOK_AGENTS: n_envs differs from the attached buffers");
+  if ((flags & CZ_STEP_KEEP_ALL) && k_steps > t->cook.k_cap)
+    return cz_fail(CZ_EINVAL, "%s", "CZ_STEP_COOK_AGENTS with CZ_STEP_KEEP_ALL: k_steps exceeds the attached k_capacity");
+  return CZ_OK;
+}
+static int cz_cook_merge(const cz_tables* t, const uint32_t* state, const uint8_t* in, uint8_t* out, int n_envs, uint64_t seed,
+                         uint64_t step, int64_t env_offset, bool first, cudaStream_t s);
+
 // In-place step of a large batch as `split` column ranges: the dynamics of range c + 1 (internal high-priority stream)
 // run under the row writer of range c (second internal stream), so only the first range's dynamics are exposed.  The
 // caller's stream forks into both and joins them again: every output is ordered on it when the call's work is done,
@@ -1760,29 +1773,29 @@ static int cz_step_one(const cz_tables* t, uint32_t* state, const uint8_t* actio
 // k_steps consecutive steps of every environment in ONE launch of the warp-per-environment kernel
 static int cz_launch_warp(const cz_tables* t, uint32_t* state, const uint8_t* actions, double* obs, double* reward,
                           uint8_t* terminated, uint8_t* truncated, uint32_t* error_flags, int n_envs, int k_steps, uint32_t flags,
-                          uint64_t seed, int64_t env_offset, uint64_t action_step, void* stream, bool stats) {
+                          uint64_t seed, int64_t env_offset, uint64_t action_step, void* stream, bool stats, bool cook) {
   if (((uintptr_t)obs & 15) != 0) return cz_fail(CZ_EINVAL, "%s", "obs must be 16-byte aligned");
   const CzDev& T = t->dev;
   // two environments per warp (16-lane groups) when every dynamic slot finds a lane in half a warp
   const int G = t->warp_group;
   const int groups = WK_WARPS * 32 / G;
   const int blocks = (n_envs + groups - 1) / groups;
-  const size_t smem = wk_smem_bytes(T.V, T.A, CZ_WARP_WHOLE ? T.L : T.stage_len, G);
+  const size_t smem = wk_smem_bytes(T.V, T.A, CZ_WARP_WHOLE ? T.L : T.stage_len, G, cook);
   cudaStream_t s = (cudaStream_t)stream;
-#define CZ_WARP_GO_S(NA, S)                                                                                                    \
+#define CZ_WARP_GO_S(NA, C, S)                                                                                                  \
   if (G == 16)                                                                                                                 \
-    cz_warp_kernel<NA, 16, S><<<blocks, 32 * WK_WARPS, smem, s>>>(t->dev, state, actions, obs, reward, terminated, truncated,   \
-                                                                  error_flags, n_envs, k_steps, flags, seed, env_offset,         \
-                                                                  action_step, t->stats);                                        \
+    cz_warp_kernel<NA, 16, C, S><<<blocks, 32 * WK_WARPS, smem, s>>>(t->dev, state, actions, obs, reward, terminated, truncated,\
+                                                                     error_flags, n_envs, k_steps, flags, seed, env_offset,      \
+                                                                     action_step, t->stats, t->cook);                            \
   else                                                                                                                         \
-    cz_warp_kernel<NA, 32, S><<<blocks, 32 * WK_WARPS, smem, s>>>(t->dev, state, actions, obs, reward, terminated, truncated,   \
-                                                                  error_flags, n_envs, k_steps, flags, seed, env_offset,         \
-                                                                  action_step, t->stats)
-#define CZ_WARP_GO(NA)          \
-  if (stats) {                  \
-    CZ_WARP_GO_S(NA, true);     \
-  } else {                      \
-    CZ_WARP_GO_S(NA, false);    \
+    cz_warp_kernel<NA, 32, C, S><<<blocks, 32 * WK_WARPS, smem, s>>>(t->dev, state, actions, obs, reward, terminated, truncated,\
+                                                                     error_flags, n_envs, k_steps, flags, seed, env_offset,      \
+                                                                     action_step, t->stats, t->cook)
+#define CZ_WARP_GO(NA)                                                   \
+  if (cook) {                                                            \
+    if (stats) { CZ_WARP_GO_S(NA, true, true); } else { CZ_WARP_GO_S(NA, true, false); }   \
+  } else {                                                               \
+    if (stats) { CZ_WARP_GO_S(NA, false, true); } else { CZ_WARP_GO_S(NA, false, false); } \
   }
   switch (T.A) {
     case 1: CZ_WARP_GO(1); break;
@@ -1811,15 +1824,21 @@ extern "C" int cz_step(const cz_tables* t, uint32_t* state, const uint8_t* actio
     if (rc != CZ_OK) return rc;
     flags &= ~CZ_STEP_EPISODE_STATS;
   }
+  const bool cook = (flags & CZ_STEP_COOK_AGENTS) != 0;
+  if (cook) {
+    int rc = cz_cook_check(t, n_envs, k_steps, flags);
+    if (rc != CZ_OK) return rc;
+    flags &= ~CZ_STEP_COOK_AGENTS;
+  }
   if (n_envs <= 0) return CZ_OK;
   const CzDev& T = t->dev;
   const bool warp_ok = (t->simple || t->simple2) && !(flags & CZ_STEP_OBS_F32);
   if (warp_ok && (k_steps > 1 ? n_envs <= t->warp_k_max_envs : n_envs <= t->warp_max_envs))
     return cz_launch_warp(t, state, actions, obs, reward, terminated, truncated, error_flags, n_envs, k_steps, flags, seed,
-                          env_offset, action_step, stream, stats);
+                          env_offset, action_step, stream, stats, cook);
   // everything else (generic tables, float32 rows, large batches): k_steps launches of the per-step kernels
   cz_tables* tm = const_cast<cz_tables*>(t);
-  if (dev_actions && n_envs > t->rand_envs) {
+  if (dev_actions && !cook && n_envs > t->rand_envs) {
     if (tm->d_rand) cudaFree(tm->d_rand);
     tm->rand_envs = 0;
     CZ_CUDA(cudaMalloc((void**)&tm->d_rand, (size_t)n_envs * T.A));
@@ -1829,12 +1848,18 @@ extern "C" int cz_step(const cz_tables* t, uint32_t* state, const uint8_t* actio
   const bool keep = (flags & CZ_STEP_KEEP_ALL) != 0 && k_steps > 1;
   const size_t obs_bytes = na * T.L * ((flags & CZ_STEP_OBS_F32) ? sizeof(float) : sizeof(double));
   for (int k = 0; k < k_steps; ++k) {
+    const size_t o = keep ? (size_t)k : 0;
     const uint8_t* a = actions ? actions + (size_t)k * na : t->d_rand;
-    if (dev_actions) {
+    if (cook) {  // the merged actions of this step into its actions_taken slice, which the dynamics then read
+      uint8_t* taken = t->cook.actions_taken + o * na;
+      int rc = cz_cook_merge(t, state, actions ? a : nullptr, taken, n_envs, seed, action_step + (uint64_t)k, env_offset, k == 0,
+                             (cudaStream_t)stream);
+      if (rc != CZ_OK) return rc;
+      a = taken;
+    } else if (dev_actions) {
       int rc = cz_random_actions(t, tm->d_rand, n_envs, seed, action_step + (uint64_t)k, env_offset, stream);
       if (rc != CZ_OK) return rc;
     }
-    const size_t o = keep ? (size_t)k : 0;
     double* obs_k = obs ? reinterpret_cast<double*>(reinterpret_cast<char*>(obs) + o * obs_bytes) : nullptr;
     // KEEP_ALL: step k's rows start k * obs_bytes into the buffer, which is 16-byte aligned only when obs_bytes is a multiple
     // of 16 (odd n * A * L in float64, n * A * L not a multiple of 4 in float32); the row writers need 16-byte aligned rows,
@@ -1950,6 +1975,12 @@ extern "C" int cz_step_pipelined(cz_tables* t, uint32_t* state2, const uint8_t* 
     if (rc != CZ_OK) return rc;
     flags &= ~CZ_STEP_EPISODE_STATS;
   }
+  const bool cook = (flags & CZ_STEP_COOK_AGENTS) != 0;
+  if (cook) {
+    int rc = cz_cook_check(t, n_envs, 1, flags);
+    if (rc != CZ_OK) return rc;
+    flags &= ~CZ_STEP_COOK_AGENTS;
+  }
   int rc = cz_pipe_init(t);
   if (rc != CZ_OK) return rc;
   const size_t half = (size_t)t->dev.rows * n_envs;
@@ -1962,6 +1993,11 @@ extern "C" int cz_step_pipelined(cz_tables* t, uint32_t* state2, const uint8_t* 
   CZ_CUDA(cudaStreamWaitEvent(t->pipe_dyn, t->ev_user, 0));
   // the observe kernel that read the half we are about to overwrite must be done
   if (t->pipe_obs_pending[nxt]) CZ_CUDA(cudaStreamWaitEvent(t->pipe_dyn, t->ev_obs[nxt], 0));
+  if (cook) {  // on the dynamics stream, after the same waits and before the dynamics that read the merged actions
+    rc = cz_cook_merge(t, in, actions, t->cook.actions_taken, n_envs, seed, 0, env_offset, true, t->pipe_dyn);
+    if (rc != CZ_OK) return rc;
+    actions = t->cook.actions_taken;
+  }
   rc = cz_launch<MODE_STEP>(t, in, out, true, actions, nullptr, nullptr, nullptr, obs, reward, terminated, truncated,
                             error_flags, n_envs, flags, seed, env_offset, t->pipe_dyn, 0,
                             t->pipe_steps == 0 ? 0 : t->pipe_dyn_blocks);  // nothing to hide behind on the first step: full grid
@@ -2014,6 +2050,7 @@ extern "C" int cz_step_host(cz_tables* t, uint32_t* state_dev, const uint8_t* ac
   if (!t || !actions_host || !obs_host || !reward_host || !terminated_host || !truncated_host)
     return cz_fail(CZ_EINVAL, "%s", "null argument");
   const CzDev& T = t->dev;
+  if (flags & CZ_STEP_COOK_AGENTS) return cz_fail(CZ_EINVAL, "%s", "cz_step_host does not take CZ_STEP_COOK_AGENTS (use cz_step)");
   if (flags & CZ_STEP_EPISODE_STATS) {
     int rc = cz_stats_check(t, n_envs);
     if (rc != CZ_OK) return rc;

@@ -700,9 +700,11 @@ __device__ __forceinline__ void wk_pair_store(const CzDev& T, const WEnv<NA, G>&
     if (k < (int)flen) *reinterpret_cast<uint2*>(out + 2 + k) = make_uint2(0u, (fb >> k & 1u) ? 0x3FF00000u : 0u);
 }
 
-__host__ __device__ inline size_t wk_smem_bytes(int V, int A, int stage_len, int G) {
+// cook: the COOK instantiation's per-group scratch of CZ_MAX_DYN slot records follows the WK_WORDS words
+__host__ __device__ inline size_t wk_smem_bytes(int V, int A, int stage_len, int G, bool cook = false) {
   const int groups = WK_WARPS * 32 / G;
-  return cz_block_smem_head(V) + 64 * 4 + (size_t)groups * (WK_WORDS * 4 + (size_t)A * ((stage_len + 1) / 2) * 16);
+  return cz_block_smem_head(V) + 64 * 4 +
+         (size_t)groups * (WK_WORDS * 4 + (cook ? CZ_MAX_DYN * 4 : 0) + (size_t)A * ((stage_len + 1) / 2) * 16);
 }
 
 // STATS (CZ_STEP_EPISODE_STATS): the episode-statistics record of the group's environment (cz_stats.cuh) is loaded in the
@@ -710,15 +712,33 @@ __host__ __device__ inline size_t wk_smem_bytes(int V, int A, int stage_len, int
 // agent g's running return, and K steps stay one launch.  STATS = false compiles to the kernel without any of it (the same
 // SASS as a kernel without the statistics code); the true instantiation has its own bound for 32-lane groups, where the plain
 // kernel's 7 blocks per SM (72 registers) spill the record.
+//
+// COOK (CZ_STEP_COOK_AGENTS): before each of the K steps the group writes its slot records to a private scratch of
+// CZ_MAX_DYN words, builds the cook's per-environment masks with group reductions, and lanes g < NA whose bit is set in the
+// environment's agent mask run pol_cook (cz_policy_dev.cuh) on that scratch; their decisions replace the caller's / the
+// stream's actions where the action word is formed.  Every step's actions go to the actions_taken slice, the raise bits
+// are ORed in registers until the epilogue, and K closed-loop steps stay one launch.  COOK = false compiles to the kernel
+// without any of it.
 #ifndef CZ_WARP_STATS_MIN_BLOCKS32
 #define CZ_WARP_STATS_MIN_BLOCKS32 6
 #endif
-template <int NA, int G, bool STATS>
-__global__ void __launch_bounds__(32 * WK_WARPS, G == 32 ? (STATS ? CZ_WARP_STATS_MIN_BLOCKS32 : 7) : 4)
+// With 32-lane groups COOK has bounds of its own: 6 blocks per SM (80 registers) alone, 5 with STATS, where 6 spilled
+// 40-52 bytes.
+#ifndef CZ_WARP_COOK_MIN_BLOCKS32
+#define CZ_WARP_COOK_MIN_BLOCKS32 6
+#endif
+#ifndef CZ_WARP_COOK_STATS_MIN_BLOCKS32
+#define CZ_WARP_COOK_STATS_MIN_BLOCKS32 5
+#endif
+template <int NA, int G, bool COOK, bool STATS>
+__global__ void __launch_bounds__(32 * WK_WARPS,
+                                  G == 32 ? (COOK ? (STATS ? CZ_WARP_COOK_STATS_MIN_BLOCKS32 : CZ_WARP_COOK_MIN_BLOCKS32)
+                                                  : (STATS ? CZ_WARP_STATS_MIN_BLOCKS32 : 7))
+                                          : 4)
 cz_warp_kernel(const __grid_constant__ CzDev T, uint32_t* __restrict__ state, const uint8_t* __restrict__ actions,
                double* __restrict__ obs, double* __restrict__ reward, uint8_t* __restrict__ term, uint8_t* __restrict__ trunc,
                uint32_t* __restrict__ errflags, int n_envs, int k_steps, uint32_t flags, uint64_t seed, int64_t env_offset,
-               uint64_t action_step, const __grid_constant__ CzStatsDev S) {
+               uint64_t action_step, const __grid_constant__ CzStatsDev S, const __grid_constant__ CzCookDev C) {
   constexpr bool FAST = true;
   constexpr int GROUPS = WK_WARPS * 32 / G;  // environments per block
   constexpr int TK = 64 / G;                 // table elements (double2) of a row per lane, at most
@@ -748,9 +768,11 @@ cz_warp_kernel(const __grid_constant__ CzDev T, uint32_t* __restrict__ state, co
     pmap[threadIdx.x] = lm.x >= 0 ? ((uint32_t)lm.x & 0x1FFFFFFu) | ((uint32_t)lm.y << 25) : 0u;
   }
   const int stage2 = CZ_WARP_WHOLE ? (T.L >> 1) : ((T.stage_len + 1) >> 1);  // double2 per staging row (whole rows or the computed span)
-  unsigned char* gsm = smem_wk + head + 256 + (size_t)grp * (WK_WORDS * 4 + (size_t)NA * stage2 * 16);
+  constexpr int COOK_BYTES = COOK ? CZ_MAX_DYN * 4 : 0;
+  unsigned char* gsm = smem_wk + head + 256 + (size_t)grp * (WK_WORDS * 4 + COOK_BYTES + (size_t)NA * stage2 * 16);
   uint32_t* wwords = reinterpret_cast<uint32_t*>(gsm);  // cells[64] | skp[8] | plist[32] uint2
-  double2* stage = reinterpret_cast<double2*>(gsm + WK_WORDS * 4);
+  uint32_t* cook_slots = reinterpret_cast<uint32_t*>(gsm + WK_WORDS * 4);  // COOK: [CZ_MAX_DYN] slot records
+  double2* stage = reinterpret_cast<double2*>(gsm + WK_WORDS * 4 + COOK_BYTES);
 #pragma unroll 1
   for (int k = g; k < NA * stage2; k += G) stage[k] = make_double2(0.0, 0.0);  // never-occupied slots stay zero
   __syncthreads();
@@ -797,6 +819,9 @@ cz_warp_kernel(const __grid_constant__ CzDev T, uint32_t* __restrict__ state, co
     st_open = S.open[env];
     if (g < NA) st_ret[0] = S.ret[(size_t)env * NA + g];
   }
+  // cook agents: the environment's mask (group-uniform), and this lane's raise bit ORed over the launch's steps
+  uint32_t cook_mask = 0, cook_bad = 0;
+  if constexpr (COOK) cook_mask = C.agent_mask[env];
 
   // where this lane's table elements (double2 units g, g + G, ...) land in a row: segment 0 first, then segment 1
   int tdst[TK];
@@ -826,6 +851,30 @@ cz_warp_kernel(const __grid_constant__ CzDev T, uint32_t* __restrict__ state, co
         const int a = (int)(u * num_actions);
         a_mine = (uint32_t)(a < num_actions ? a : num_actions - 1);
       }
+    }
+    if constexpr (COOK) {
+      // cz_policy_act on the state before this step (on an auto-reset step the finished one, whose decision the reset ignores)
+      if (cook_mask) {
+        if (g < D) cook_slots[g] = e.rec;
+        PolEnv pe;
+        const uint64_t fb = pol_fills(e.rec) ? 1ull << O_XY(e.rec) : 0ull;
+        pe.filled = (uint64_t)g_or(e, (uint32_t)fb) | ((uint64_t)g_or(e, (uint32_t)(fb >> 32)) << 32);
+        g_sync(e);
+        if (g < NA && (cook_mask >> g & 1u)) {
+          pol_app_masks(C.P, e.variant, pe);
+          // cook g follows recipe g of its environment unless told otherwise: the step's marks are then those of its graph
+          const uint32_t rid = C.cook_recipes ? C.cook_recipes[(size_t)env * NA + g] : ((e.rids >> (8 * g)) & 255u);
+          const uint32_t marks = (!C.cook_recipes && g < T.R && C.P.use_env_marks) ? ((e.marks >> (8 * g)) & 255u) : 0x100u;
+          bool crash = false;
+          uint32_t a = 0;
+          if (rid < (uint32_t)T.B) a = pol_cook<1>(T, C.P, pe, cook_slots, e.variant, wk_sel(e.ag, g), rid, marks, crash);
+          else crash = true;
+          if (crash) cook_bad |= 1u << g;
+          a_mine = crash ? 0u : a;
+        }
+        g_sync(e);  // the scratch is rewritten by the next step
+      }
+      if (g < NA) C.actions_taken[((keep ? (size_t)k : 0) * N + env) * NA + g] = (uint8_t)a_mine;
     }
     uint32_t act = 0;
 #pragma unroll
@@ -955,6 +1004,10 @@ cz_warp_kernel(const __grid_constant__ CzDev T, uint32_t* __restrict__ state, co
     state[(size_t)(D + g) * N + env] = w;
   }
   if (errflags && e.err && g == 0) errflags[env] |= e.err;
+  if constexpr (COOK) {
+    const uint32_t bad = g_or(e, cook_bad);
+    if (C.crashed && g == 0) C.crashed[env] = (uint8_t)bad;
+  }
   if constexpr (STATS) {
     if (g < NA) S.ret[(size_t)env * NA + g] = st_ret[0];
     if (g == 0) {

@@ -21,6 +21,9 @@ class MixedAgentCookingEnv:
         if any(o == "grid" for o in kwargs.get("obs_spaces") or ()):
             # the grid's channel count grows with the agent count: the groups would not share one observation shape
             raise NotImplementedError("MixedAgentCookingEnv builds feature_vector observations only")
+        if kwargs.get("cook_agents") is not None:
+            # agent indices mean different agents in groups of different sizes
+            raise NotImplementedError("cook_agents is not supported by MixedAgentCookingEnv")
         counts = np.asarray(agent_counts, dtype=np.int64)
         if counts.ndim != 1 or counts.size == 0 or counts.min() < 1:
             raise ValueError("agent_counts must be a non-empty vector of positive agent counts")

@@ -94,6 +94,34 @@ extern "C" {
 #define CZ_STEP_EPISODE_STATS 16u /* update the episode statistics attached with cz_stats_attach after every step of every
                                   environment (honoured by cz_step, cz_step_pipelined and cz_step_host; CZ_EINVAL when no
                                   statistics are attached or their n_envs differs from the call's) */
+#define CZ_STEP_COOK_AGENTS 32u   /* agents in the attached mask act by the device cook (cz_cook_attach); rule below */
+
+/* ---- cook agents (CZ_STEP_COOK_AGENTS) -----------------------------------------------------------------------------
+ * For every environment e and every step k of a call with the flag set:
+ *   1. on the state BEFORE the step, every agent i whose bit is set in agent_mask[e] gets the action cz_policy_act would
+ *      return for it (following cook_recipes[e][i], or recipe i of the environment when cook_recipes is NULL); a cook that
+ *      would raise acts 0 and sets bit i of crashed[e];
+ *   2. every other agent gets the action the step would have used anyway: actions[k][e][i], or under
+ *      CZ_STEP_DEVICE_ACTIONS the draw of the counter stream at step index action_step + k;
+ *   3. the step runs exactly as cz_step does with those actions, and they are written to actions_taken (slice k under
+ *      CZ_STEP_KEEP_ALL, slice 0 otherwise).
+ * So every path gives, bit for bit, the composition cz_policy_act -> overwrite the masked columns -> cz_step(k_steps = 1),
+ * one step at a time: state, rows, rewards, flags, error_flags and episode statistics.  On an auto-reset step the decision
+ * is taken on the finished state and then ignored by the reset.  crashed is overwritten by each call with the OR of its
+ * steps' raise bits (masked agents only).  Honoured by cz_step (one more launch per step on the per-step kernels; K steps
+ * of the warp kernel stay one launch) and cz_step_pipelined (k = 0, no DEVICE_ACTIONS); cz_step_host returns CZ_EINVAL.
+ * CZ_EINVAL as well: the flag with nothing attached, an n_envs different from the attached one (n_envs = 0 included, as
+ * for CZ_STEP_EPISODE_STATS: the flag is checked before the empty batch returns), and CZ_STEP_KEEP_ALL with
+ * k_steps > k_capacity. */
+typedef struct cz_cook_desc {
+  int32_t n_envs;
+  int32_t k_capacity;          /* steps actions_taken holds (>= 1)                                                     */
+  const uint8_t* agent_mask;   /* [n] bit i: agent i of the environment is driven by the cook                          */
+  const uint8_t* cook_recipes; /* [n][A] book index each cook follows, or NULL: cook i follows recipe i                */
+  uint8_t* actions_taken;      /* [k_capacity][n][A] the actions each step applied (slice k under CZ_STEP_KEEP_ALL,
+                                  slice 0 otherwise)                                                                    */
+  uint8_t* crashed;            /* [n] or NULL: OR over the call's steps of the cook's raise bits                        */
+} cz_cook_desc;
 
 /* ---- episode statistics ----------------------------------------------------------------------
  * Every environment carries a record (cz_stats_desc).  After each step of the environment, with the post-step rows EPISODE,
@@ -347,6 +375,12 @@ int cz_policy_act(const cz_policy* p, const uint32_t* state, const uint8_t* cook
  * of an environment does not depend on the batch it is stepped in. */
 int cz_random_actions(const cz_tables* t, uint8_t* actions, int n_envs, uint64_t seed, uint64_t step,
                       int64_t env_offset, void* stream);
+
+/* Attach caller-owned device buffers and the policy for CZ_STEP_COOK_AGENTS (d == NULL detaches).  CZ_EINVAL for a policy
+ * created from other tables, a NULL agent_mask or actions_taken, n_envs < 1 or k_capacity < 1.  Host-side bookkeeping
+ * only (no kernel, no synchronisation): re-attaching between calls, e.g. a fresh [K][n][A] actions_taken per call, is
+ * cheap and legal under stream capture.  The tables keep the pointers: buffers and policy must outlive the attachment. */
+int cz_cook_attach(cz_tables* t, const cz_policy* p, const cz_cook_desc* d);
 
 /* Number of kernels launched by this library since load (the bench's gpu_launches claim). */
 uint64_t cz_launch_count(void);
