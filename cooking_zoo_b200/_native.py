@@ -77,6 +77,8 @@ SIGNATURES = {
     "cz_observe_f32": (C.c_int, [_P, _P, _P, C.c_int, _P]),
     "cz_grid_channels": (C.c_int, [_P]),
     "cz_observe_grid": (C.c_int, [_P, _P, _P, C.c_int, _P]),
+    "cz_observe_agents": (C.c_int, [_P, _P, C.c_uint32, _P, C.c_uint32, C.c_int, _P]),
+    "cz_observe_grid_agents": (C.c_int, [_P, _P, C.c_uint32, _P, C.c_int, _P]),
     "cz_step_pipelined": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, C.c_int, C.c_uint32, C.c_uint64, C.c_int64, _P]),
     "cz_pipeline_config": (C.c_int, [_P, C.c_int, C.c_int]),
     "cz_pipeline_wait": (C.c_int, [_P, _P]),

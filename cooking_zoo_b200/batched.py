@@ -47,7 +47,7 @@ class BatchedCookingEnv:
                  device="cuda:0", recipe_pool=None, layout_pool_size="auto", layout_seed=0, layouts=None,
                  auto_reset=False, seed=0, env_offset=0, pipelined=False, obs_dtype=torch.float64, stream=None,
                  pipeline_buffers=2, background_dynamics=0, background_policy=0, episode_stats=False, cook_agents=None,
-                 cook_recipes=None):
+                 cook_recipes=None, obs_agents=None):
         obs_spaces = obs_spaces or ["feature_vector"] * num_agents
         if obs_spaces and all(o == "grid" for o in obs_spaces):
             # per-cell u8 planes [N, A, C, H, W] written by their own kernel after the dynamics (cooking_zoo_b200.grid)
@@ -107,12 +107,20 @@ class BatchedCookingEnv:
         if self.lib.cz_grid_channels(self._handle) != len(self.grid_channels):
             raise _native.NativeError("libcz_b200.so and cooking_zoo_b200.grid disagree on the grid's channels")
         self._grid_shape = (N, A, len(self.grid_channels), t.height, t.width)
+        # observations of the agents in obs_agents only: row / block j belongs to agent obs_agents[j] (cz_observe_agents)
+        self.obs_agents = self._check_obs_agents(obs_agents)
+        M = len(self.obs_agents)
+        self._obs_mask = sum(1 << a for a in self.obs_agents)
+        if M < A and self.pipelined:
+            raise NotImplementedError("obs_agents: the pipelined step writes every agent's rows on its internal stream")
         if self.obs_mode == "grid":
-            self.obs = torch.zeros(self._grid_shape, dtype=torch.uint8, device=dev)
-            # chosen once here, so that the feature-vector methods keep their host code unchanged
-            self.__class__ = _GridModeEnv
+            self.obs = torch.zeros((N, M) + self._grid_shape[2:], dtype=torch.uint8, device=dev)
         else:
-            self.obs = torch.zeros((N, A, L), dtype=obs_dtype, device=dev)
+            self.obs = torch.zeros((N, M, L), dtype=obs_dtype, device=dev)
+        if self.obs_mode == "grid" or M < A:
+            # dynamics without rows, then the observation writer (_writer); chosen once here, so that the methods of full
+            # feature-vector rows keep their host code unchanged
+            self.__class__ = _WriterEnv
         self.reward = torch.zeros((N, A), dtype=torch.float64, device=dev)
         self.terminated = torch.zeros((N, A), dtype=torch.uint8, device=dev)
         self.truncated = torch.zeros((N, A), dtype=torch.uint8, device=dev)
@@ -129,6 +137,22 @@ class BatchedCookingEnv:
             self._attach_cook(cook_agents, cook_recipes)
         elif cook_recipes is not None:
             raise ValueError("cook_recipes applies to the agents named by cook_agents")
+
+    def _check_obs_agents(self, obs_agents):
+        """obs_agents (None: every agent) -> tuple of distinct agent indices in ascending order"""
+        A = self.num_agents
+        if obs_agents is None:
+            return tuple(range(A))
+        idx = [int(i) for i in obs_agents]
+        if not idx:
+            raise ValueError("obs_agents must name at least one agent")
+        if len(set(idx)) != len(idx):
+            raise ValueError("obs_agents must not name an agent twice")
+        if any(i < 0 or i >= A for i in idx):
+            raise ValueError(f"obs_agents: agent indices must lie in 0..{A - 1}")
+        if idx != sorted(idx):
+            raise ValueError("obs_agents must list the agents in ascending order (observation j is agent obs_agents[j])")
+        return tuple(idx)
 
     def _attach_cook(self, cook_agents, cook_recipes):
         """agents driven by the device cook inside every step (CZ_STEP_COOK_AGENTS, cz_cook_attach)"""
@@ -288,7 +312,7 @@ class BatchedCookingEnv:
             mk = torch.as_tensor(mask).to(torch.uint8).to(self.device).contiguous()
         with torch.cuda.device(self.device):
             f32 = self.obs_dtype == torch.float32
-            grid = self.obs_mode == "grid"
+            written = isinstance(self, _WriterEnv)
             if self.pipelined:
                 # drain the internal streams (dynamics / row writer still in flight) and keep stepping from the half
                 # that holds the current state: a masked reset must land next to the untouched environments
@@ -298,12 +322,11 @@ class BatchedCookingEnv:
             _native.check(self.lib.cz_reset(self._handle, self.state.data_ptr(), lid.data_ptr(),
                                             rid.data_ptr() if rid is not None else None,
                                             mk.data_ptr() if mk is not None else None,
-                                            None if f32 or grid else self.obs.data_ptr(), self.error_flags.data_ptr(),
+                                            None if f32 or written else self.obs.data_ptr(), self.error_flags.data_ptr(),
                                             N, self._stream()))
-            if grid:
-                _native.check(self.lib.cz_observe_grid(self._handle, self.state.data_ptr(), self.obs.data_ptr(), N,
-                                                       self._stream()))
-            if f32:
+            if written:
+                self._call(*self._writer(self.obs.data_ptr(), self._stream()))
+            elif f32:
                 _native.check(self.lib.cz_observe_f32(self._handle, self.state.data_ptr(), self.obs.data_ptr(), N,
                                                       self._stream()))
         return self.obs
@@ -372,9 +395,22 @@ class BatchedCookingEnv:
                                            self.seed, self.env_offset, int(action_step), self._stream()))
         return obs, rew, term, trunc, self._info
 
-    def _step_grid(self, actions):
-        """step() of grid mode: the dynamics (cz_step without observation rows), then the grid writer.
-        Returns (obs u8 [N, A, C, H, W], reward, terminated, truncated, info)."""
+    def _writer(self, out, s):
+        """(library function, arguments) writing the observation of grid mode or of an obs_agents subset from the current
+        state into device address `out` on stream `s`"""
+        h, st, N = self._handle, self.state.data_ptr(), self.num_envs
+        full = self._obs_mask == (1 << self.num_agents) - 1
+        if self.obs_mode == "grid":
+            if full:
+                return self.lib.cz_observe_grid, h, st, out, N, s
+            return self.lib.cz_observe_grid_agents, h, st, self._obs_mask, out, N, s
+        f32 = _native.STEP_OBS_F32 if self.obs_dtype == torch.float32 else 0
+        return self.lib.cz_observe_agents, h, st, self._obs_mask, out, f32, N, s
+
+    def _step_written(self, actions):
+        """step() of grid mode and of obs_agents subsets: the dynamics (cz_step without observation rows), then the
+        observation writer (_writer).  Returns (obs, reward, terminated, truncated, info); obs is u8 [N, M, C, H, W] in grid
+        mode, [N, M, L] rows otherwise (M = len(obs_agents))."""
         a = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions))
         if a.shape != self._shape_actions:
             raise ValueError("actions must have shape [num_envs, num_agents]")
@@ -386,15 +422,16 @@ class BatchedCookingEnv:
         s = self._stream()
         self._call(self.lib.cz_step, self._handle, self.state.data_ptr(), a.data_ptr(), None, self.reward.data_ptr(),
                    self.terminated.data_ptr(), self.truncated.data_ptr(), self.error_flags.data_ptr(), self.num_envs, 1,
-                   self._flags, self.seed, self.env_offset, 0, s)
-        self._call(self.lib.cz_observe_grid, self._handle, self.state.data_ptr(), self.obs.data_ptr(), self.num_envs, s)
+                   self._flags & ~_native.STEP_OBS_F32, self.seed, self.env_offset, 0, s)
+        self._call(*self._writer(self.obs.data_ptr(), s))
         return self.obs, self.reward, self.terminated, self.truncated, self._info
 
-    def _step_k_grid(self, k_steps, actions=None, action_step=0, keep_all=False):
-        """step_k() of grid mode.  keep_all=False: one cz_step of k_steps without observation rows, then one grid write.
-        keep_all=True: k single steps, each followed by its grid write into a fresh [k_steps, N, A, C, H, W] tensor."""
+    def _step_k_written(self, k_steps, actions=None, action_step=0, keep_all=False):
+        """step_k() of grid mode and of obs_agents subsets.  keep_all=False: one cz_step of k_steps without observation
+        rows, then one observation write.  keep_all=True: k single steps, each followed by its observation write into slice
+        k of a fresh [k_steps, *obs.shape] tensor."""
         N, A, K = self.num_envs, self.num_agents, int(k_steps)
-        flags = self._flags
+        flags = self._flags & ~_native.STEP_OBS_F32      # no rows from the step itself: the writer follows
         if actions is None:
             flags |= _native.STEP_DEVICE_ACTIONS
         else:
@@ -413,9 +450,9 @@ class BatchedCookingEnv:
                                                None, self.reward.data_ptr(), self.terminated.data_ptr(),
                                                self.truncated.data_ptr(), self.error_flags.data_ptr(), N, K, flags, self.seed,
                                                self.env_offset, int(action_step), s))
-                _native.check(self.lib.cz_observe_grid(self._handle, self.state.data_ptr(), self.obs.data_ptr(), N, s))
+                self._call(*self._writer(self.obs.data_ptr(), s))
                 return self.obs, self.reward, self.terminated, self.truncated, self._info
-            obs = torch.empty((K,) + self._grid_shape, dtype=torch.uint8, device=self.device)
+            obs = torch.empty((K,) + tuple(self.obs.shape), dtype=self.obs.dtype, device=self.device)
             rew = torch.empty((K, N, A), dtype=torch.float64, device=self.device)
             term = torch.empty((K, N, A), dtype=torch.uint8, device=self.device)
             trunc = torch.empty((K, N, A), dtype=torch.uint8, device=self.device)
@@ -429,7 +466,7 @@ class BatchedCookingEnv:
                                                None if actions is None else a[j].data_ptr(), None, rew[j].data_ptr(),
                                                term[j].data_ptr(), trunc[j].data_ptr(), self.error_flags.data_ptr(), N, 1,
                                                flags, self.seed, self.env_offset, int(action_step) + j, s))
-                _native.check(self.lib.cz_observe_grid(self._handle, self.state.data_ptr(), obs[j].data_ptr(), N, s))
+                self._call(*self._writer(obs[j].data_ptr(), s))
                 if cook and j > 0:
                     with torch.cuda.stream(self.stream if self.stream is not None else torch.cuda.current_stream(self.device)):
                         self.cook_step_crashed |= crash_j
@@ -438,10 +475,9 @@ class BatchedCookingEnv:
                 self.actions_taken = taken
         return obs, rew, term, trunc, self._info
 
-    def _observe_grid(self):
+    def _observe_written(self):
         with torch.cuda.device(self.device):
-            _native.check(self.lib.cz_observe_grid(self._handle, self.state.data_ptr(), self.obs.data_ptr(),
-                                                   self.num_envs, self._stream()))
+            self._call(*self._writer(self.obs.data_ptr(), self._stream()))
         return self.obs
 
     def grid_observation(self, out=None):
@@ -721,8 +757,9 @@ class BatchedCookingEnv:
         self.state[:, env] = torch.from_numpy(col.astype(np.int32)).to(self.device)
 
 
-class _GridModeEnv(BatchedCookingEnv):
-    """A BatchedCookingEnv constructed with obs_spaces=["grid"] * num_agents: step / step_k / observe write the grid."""
-    step = BatchedCookingEnv._step_grid
-    step_k = BatchedCookingEnv._step_k_grid
-    observe = BatchedCookingEnv._observe_grid
+class _WriterEnv(BatchedCookingEnv):
+    """A BatchedCookingEnv constructed with obs_spaces=["grid"] * num_agents or with obs_agents naming fewer than all agents:
+    step / step_k / observe run the dynamics without rows, then the observation writer."""
+    step = BatchedCookingEnv._step_written
+    step_k = BatchedCookingEnv._step_k_written
+    observe = BatchedCookingEnv._observe_written

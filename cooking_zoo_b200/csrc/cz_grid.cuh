@@ -28,20 +28,23 @@ struct CzGridDev {
   const uint32_t* slot_ch;    // [D] per device slot: n channel | chopped channel << 8 | mashed channel << 16 (0: none)
 };
 
-template <int NA>
-__global__ void __launch_bounds__(32 * GRID_WARPS)
-cz_grid_kernel(const __grid_constant__ CzGridDev G, const uint32_t* __restrict__ state, uint8_t* __restrict__ out, int n_envs,
-               int warps) {
+// SUB: only the observers in `mask` (ascending) get their [C][H][W] block, M = popcount(mask) blocks per environment; block j
+// is the one the full grid gives observer mask's j-th agent.  SUB = false is the full grid (mask unused).  `tid` and `bdim` are
+// threadIdx.x and blockDim.x read in the kernel itself, where the compiler knows their range from the launch bounds.
+template <int NA, bool SUB>
+__device__ __forceinline__ void cz_grid_body(const CzGridDev& G, const uint32_t* __restrict__ state, uint8_t* __restrict__ out,
+                                             int n_envs, int warps, uint32_t mask, const unsigned tid, const unsigned bdim) {
   extern __shared__ __align__(16) unsigned char gsm[];
   const unsigned full = 0xffffffffu;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int warp = tid >> 5, lane = tid & 31;
   const int e0 = blockIdx.x * warps;
   const int nb = n_envs - e0 < warps ? n_envs - e0 : warps;
-  const uint32_t E = G.E, bytes = (uint32_t)nb * E;
+  const int M = SUB ? __popc(mask) : NA;  // observer blocks per environment
+  const uint32_t E = SUB ? (uint32_t)(M * G.C * G.HW) : G.E, bytes = (uint32_t)nb * E;
   uint8_t* gbeg = out + (size_t)e0 * E;                        // the block's bytes: [gbeg, gbeg + bytes)
   const uint32_t mis = (uint32_t)((uintptr_t)gbeg & 15u);      // gsm[mis + k] is gbeg[k]
   const uint32_t span = (mis + bytes + 15u) & ~15u;
-  for (uint32_t i = threadIdx.x * 16u; i < span; i += blockDim.x * 16u) *reinterpret_cast<uint4*>(gsm + i) = make_uint4(0, 0, 0, 0);
+  for (uint32_t i = tid * 16u; i < span; i += bdim * 16u) *reinterpret_cast<uint4*>(gsm + i) = make_uint4(0, 0, 0, 0);
   const int env = e0 + warp;
   const bool live = warp < nb;
   uint32_t w0 = 0, w1 = 0;  // state rows `lane` and `lane + 32` of this warp's environment (rows <= 32 + 4 + 6)
@@ -67,6 +70,7 @@ cz_grid_kernel(const __grid_constant__ CzGridDev G, const uint32_t* __restrict__
       const bool on = kind == ST_BLENDER && (sb >> (8 + sp) & 1u);
 #pragma unroll
       for (int a = 0; a < NA; ++a) {
+        if (SUB && a >= M) break;
         uint8_t* p = b + a * CHW + c;
         p[k * HW] = 1;
         if (s0) p[ks * HW] = 1;
@@ -92,20 +96,22 @@ cz_grid_kernel(const __grid_constant__ CzGridDev G, const uint32_t* __restrict__
           const uint8_t n = (uint8_t)__popc(m);
           uint8_t* p = b + (key[j] >> 6) * HW + (key[j] & 63u);
 #pragma unroll
-          for (int a = 0; a < NA; ++a) p[a * CHW] = n;
+          for (int a = 0; a < NA; ++a)
+            if (!SUB || a < M) p[a * CHW] = n;
         }
       }
     }
-    // agent groups: lane = observer * NA + group; group 0 is the observer, then the other agents in ascending index
+    // agent groups: lane = observer block * NA + group; group 0 is the observer, then the other agents in ascending index
     {
-      const int a = lane / NA, g = lane - a * NA;
+      const int j = lane / NA, g = lane - j * NA;
+      const int a = SUB ? (j < M ? (int)__fns(mask, 0, j + 1) : 0) : j;  // the observer of block j
       const int i = g == 0 ? a : (g <= a ? g - 1 : g);
       const int src = G.D + (i < NA ? i : 0);
       const uint32_t v0 = __shfl_sync(full, w0, src & 31), v1 = __shfl_sync(full, w1, src & 31);
       const uint32_t r = src < 32 ? v0 : v1;
       const int x = r & 7u, y = (r >> 3) & 7u, o = (r >> 6) & 7u;
-      if (lane < NA * NA && x < W && y < G.H) {
-        uint8_t* p = b + a * CHW + (G.G0 + 7 * g) * HW + y * W + x;
+      if (lane < M * NA && x < W && y < G.H) {
+        uint8_t* p = b + j * CHW + (G.G0 + 7 * g) * HW + y * W + x;
         p[0] = 1;
         if (o >= 1 && o <= 4) p[o * HW] = 1;
         if (r >> 9 & 1u) p[5 * HW] = 1;
@@ -119,15 +125,30 @@ cz_grid_kernel(const __grid_constant__ CzGridDev G, const uint32_t* __restrict__
   const uintptr_t g0 = (uintptr_t)gbeg, g1 = g0 + bytes;
   const uintptr_t a0 = (g0 + 15u) & ~(uintptr_t)15u, a1 = g1 & ~(uintptr_t)15u;
   const uintptr_t head_end = a0 < g1 ? a0 : g1, tail_beg = a1 > head_end ? a1 : head_end;
-  if (threadIdx.x == 0 && a1 > a0) {
+  if (tid == 0 && a1 > a0) {
     cz_bulk_store_stream(reinterpret_cast<void*>(a0), gsm + (a0 - g0 + mis), (uint32_t)(a1 - a0));
     cz_bulk_commit();
   }
-  const int t = threadIdx.x;
+  const int t = tid;
   if (t < 16 && g0 + t < head_end) gbeg[t] = gsm[mis + t];
   if (t >= 16 && t < 32 && tail_beg + (t - 16) < g1) {
     const uintptr_t p = tail_beg + (t - 16);
     *reinterpret_cast<uint8_t*>(p) = gsm[p - g0 + mis];
   }
-  if (threadIdx.x == 0 && a1 > a0) cz_bulk_wait_read<0>();  // the staging bytes must outlive the read
+  if (tid == 0 && a1 > a0) cz_bulk_wait_read<0>();  // the staging bytes must outlive the read
+}
+
+template <int NA>
+__global__ void __launch_bounds__(32 * GRID_WARPS)
+cz_grid_kernel(const __grid_constant__ CzGridDev G, const uint32_t* __restrict__ state, uint8_t* __restrict__ out, int n_envs,
+               int warps) {
+  cz_grid_body<NA, false>(G, state, out, n_envs, warps, 0u, threadIdx.x, blockDim.x);
+}
+
+// The grid of the observers in `mask` only (cz_observe_grid_agents): [n][M][C][H][W]
+template <int NA>
+__global__ void __launch_bounds__(32 * GRID_WARPS)
+cz_grid_agents_kernel(const __grid_constant__ CzGridDev G, const uint32_t* __restrict__ state, uint8_t* __restrict__ out, int n_envs,
+                      int warps, uint32_t mask) {
+  cz_grid_body<NA, true>(G, state, out, n_envs, warps, mask, threadIdx.x, blockDim.x);
 }

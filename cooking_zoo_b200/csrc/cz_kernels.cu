@@ -1114,6 +1114,7 @@ static size_t cz_smem_bytes(const CzDev& T) {
 
 #include "cz_obs32.cuh"
 #include "cz_warp.cuh"
+#include "cz_obs_agents.cuh"
 
 extern "C" int cz_abi_version(void) { return CZ_ABI_VERSION; }
 extern "C" const char* cz_last_error(void) { return g_err; }
@@ -1387,6 +1388,7 @@ extern "C" int cz_tables_create(const cz_table_desc* d, int device, cz_tables** 
   SET_SMEM((cz_warp_kernel<4, 16, C, S>)); SET_SMEM((cz_warp_kernel<1, 32, C, S>)); SET_SMEM((cz_warp_kernel<2, 32, C, S>));    \
   SET_SMEM((cz_warp_kernel<3, 32, C, S>)); SET_SMEM((cz_warp_kernel<4, 32, C, S>))
   SET_WARP(false, false); SET_WARP(false, true); SET_WARP(true, false); SET_WARP(true, true);
+  CZ_AGENTS_INSTANCES(SET_SMEM, double); CZ_AGENTS_INSTANCES(SET_SMEM, float);
 #undef SET_WARP
 #undef SET_MODE
 #undef SET_SMEM
@@ -1916,6 +1918,50 @@ extern "C" int cz_observe_grid(const cz_tables* t, const uint32_t* state, uint8_
     case 2: cz_grid_kernel<2><<<blocks, 32 * warps, smem, s>>>(G, state, grid, n_envs, warps); break;
     case 3: cz_grid_kernel<3><<<blocks, 32 * warps, smem, s>>>(G, state, grid, n_envs, warps); break;
     default: cz_grid_kernel<4><<<blocks, 32 * warps, smem, s>>>(G, state, grid, n_envs, warps); break;
+  }
+  g_launches.fetch_add(1);
+  CZ_CUDA(cudaGetLastError());
+  return CZ_OK;
+}
+
+// ---- observations of chosen agents (cz_observe_agents, cz_observe_grid_agents) ----
+static int cz_agents_check(const cz_tables* t, const uint32_t* state, uint32_t agent_mask, const void* out) {
+  if (!t || !state || !out) return cz_fail(CZ_EINVAL, "%s", "null argument");
+  if (agent_mask == 0 || (agent_mask >> t->dev.A) != 0)
+    return cz_fail(CZ_EINVAL, "%s", "agent_mask must name at least one agent and no agent at or above num_agents");
+  return CZ_OK;
+}
+
+extern "C" int cz_observe_agents(const cz_tables* t, const uint32_t* state, uint32_t agent_mask, void* obs, uint32_t flags,
+                                 int n_envs, void* stream) {
+  int rc = cz_agents_check(t, state, agent_mask, obs);
+  if (rc != CZ_OK) return rc;
+  if (flags & ~CZ_STEP_OBS_F32) return cz_fail(CZ_EINVAL, "%s", "cz_observe_agents takes no flag but CZ_STEP_OBS_F32");
+  const bool f32 = (flags & CZ_STEP_OBS_F32) != 0;
+  if (((uintptr_t)obs & (f32 ? 3 : 7)) != 0) return cz_fail(CZ_EINVAL, "%s", "obs must be aligned to its element size");
+  if (n_envs <= 0) return CZ_OK;
+  if (f32) return cz_launch_obs_agents(t, state, reinterpret_cast<float*>(obs), agent_mask, n_envs, (cudaStream_t)stream);
+  return cz_launch_obs_agents(t, state, reinterpret_cast<double*>(obs), agent_mask, n_envs, (cudaStream_t)stream);
+}
+
+extern "C" int cz_observe_grid_agents(const cz_tables* t, const uint32_t* state, uint32_t agent_mask, uint8_t* grid, int n_envs,
+                                      void* stream) {
+  int rc = cz_agents_check(t, state, agent_mask, grid);
+  if (rc != CZ_OK) return rc;
+  if (n_envs <= 0) return CZ_OK;
+  const CzGridDev& G = t->grid;
+  const size_t E = (size_t)__builtin_popcount(agent_mask) * G.C * G.HW;  // bytes per environment
+  int warps = (int)(GRID_SMEM_BUDGET / E);
+  if (warps > GRID_WARPS) warps = GRID_WARPS;
+  if (warps < 1) warps = 1;
+  const size_t smem = ((size_t)warps * E + 30) & ~(size_t)15;  // up to 15 bytes of shift in front, rounded up to 16
+  const int blocks = (n_envs + warps - 1) / warps;
+  cudaStream_t s = (cudaStream_t)stream;
+  switch (t->dev.A) {
+    case 1: cz_grid_agents_kernel<1><<<blocks, 32 * warps, smem, s>>>(G, state, grid, n_envs, warps, agent_mask); break;
+    case 2: cz_grid_agents_kernel<2><<<blocks, 32 * warps, smem, s>>>(G, state, grid, n_envs, warps, agent_mask); break;
+    case 3: cz_grid_agents_kernel<3><<<blocks, 32 * warps, smem, s>>>(G, state, grid, n_envs, warps, agent_mask); break;
+    default: cz_grid_agents_kernel<4><<<blocks, 32 * warps, smem, s>>>(G, state, grid, n_envs, warps, agent_mask); break;
   }
   g_launches.fetch_add(1);
   CZ_CUDA(cudaGetLastError());

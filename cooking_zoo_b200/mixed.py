@@ -24,6 +24,9 @@ class MixedAgentCookingEnv:
         if kwargs.get("cook_agents") is not None:
             # agent indices mean different agents in groups of different sizes
             raise NotImplementedError("cook_agents is not supported by MixedAgentCookingEnv")
+        if kwargs.get("obs_agents") is not None:
+            # agent indices mean different agents in groups of different sizes
+            raise NotImplementedError("obs_agents is not supported by MixedAgentCookingEnv")
         counts = np.asarray(agent_counts, dtype=np.int64)
         if counts.ndim != 1 or counts.size == 0 or counts.min() < 1:
             raise ValueError("agent_counts must be a non-empty vector of positive agent counts")

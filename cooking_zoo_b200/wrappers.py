@@ -53,6 +53,9 @@ class ParallelCookingEnv:
     def __init__(self, level, meta_file, num_agents, max_steps, recipes, agent_visualization=None, obs_spaces=None,
                  end_condition_all_dishes=False, action_scheme="scheme1", render=False, reward_scheme=None,
                  agent_respawn_rate=0.0, grace_period=20, agent_despawn_rate=0.0, **backend_kwargs):
+        if backend_kwargs.get("obs_agents") is not None:
+            # the PettingZoo / gym APIs hand every agent its own observation
+            raise NotImplementedError("obs_agents is not supported by the PettingZoo / gym wrappers")
         self._b = BatchedCookingEnv(1, level, meta_file, num_agents, max_steps, recipes, agent_visualization,
                                     obs_spaces, end_condition_all_dishes, action_scheme, render, reward_scheme,
                                     agent_respawn_rate, grace_period, agent_despawn_rate, **backend_kwargs)

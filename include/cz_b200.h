@@ -285,6 +285,25 @@ int cz_grid_channels(const cz_tables* t);
 /* grid of every environment from the current state, asynchronous on `stream`; no alignment requirement on `grid`. */
 int cz_observe_grid(const cz_tables* t, const uint32_t* state, uint8_t* grid, int n_envs, void* stream);
 
+/* ---- observations of chosen agents ---------------------------------------------------------
+ * For a learner among scripted partners (CZ_STEP_COOK_AGENTS), or one policy evaluated against fixed ones, only some agents'
+ * observations are read.  Let M = popcount(agent_mask) and a_j the j-th set bit of agent_mask (ascending).  Then, element for
+ * element and bit for bit:
+ *   cz_observe_agents       obs [n][M][L]: row j of environment e is row a_j of environment e that cz_observe writes (float64),
+ *                           or that cz_observe_f32 writes under flags = CZ_STEP_OBS_F32;
+ *   cz_observe_grid_agents  grid u8 [n][M][C][H][W]: block j of environment e is the [C][H][W] block cz_observe_grid writes for
+ *                           observer a_j (its agent groups in the same order: a_j first, then the others ascending).
+ * A step that writes only these is cz_step with obs == NULL (cz_reset with obs == NULL), then one of these calls on the same
+ * stream.  Both return CZ_EINVAL for a NULL t / state / output, an agent_mask of 0 or with a bit at or above num_agents, and
+ * (cz_observe_agents) a flag other than CZ_STEP_OBS_F32; n_envs <= 0 launches nothing.
+ * Alignment: `obs` needs the alignment of its element (8 bytes for float64, 4 for float32) and nothing more, so every slice
+ * of a [K][n][M][L] buffer works; a 16-byte aligned `obs` takes the bulk-store writer of the packed plans.  `grid` has no
+ * alignment requirement. */
+int cz_observe_agents(const cz_tables* t, const uint32_t* state, uint32_t agent_mask, void* obs, uint32_t flags, int n_envs,
+                      void* stream);
+int cz_observe_grid_agents(const cz_tables* t, const uint32_t* state, uint32_t agent_mask, uint8_t* grid, int n_envs,
+                           void* stream);
+
 /* The reference-facing call with HOST buffers: copies actions host->device, steps, copies
  * obs/reward/flags device->host, and synchronises the stream before returning.  Scratch
  * device buffers are owned by the tables object (sized on first use). */
